@@ -7,7 +7,7 @@ one batch of synthetic item sets, n_hidden 100, n_code 50.  The headline workloa
 configuration (configs[1]) and the other configs are extra legs of the same JSON line.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu]
-                  [--workload mpd|pubmed|econbiz]
+                  [--workload mpd|pubmed|econbiz] [--dump-outputs DIR]
 
 Prints ONE JSON line.  ``value`` = sets/s with the batches already resident in HBM (device-timed with CUDA events,
 exactly K steps, max over ranks); ``e2e`` = the same through the host-buffer entry ``partial_fit`` calls (pinned CSR
@@ -20,7 +20,13 @@ DESIGN.md 4); the predict legs carry ``cpu_baseline`` = the reference's predict 
 host cores (internal ``--impl reference-predict``).
 
 ``--impl reference`` times the reference's CPU path alone (rank 0 only) and prints the same line with
-``"impl": "reference"``.
+``"impl": "reference"``.  ``--steps K`` is exactly the number of timed steps of ``--impl ours``; the reference arm runs
+at most K and stops earlier once ``--budget`` seconds of timed work are spent (its CPU-port fallback without the
+reference package: at most 20), and reports the steps it timed in ``steps_timed``.
+
+``--dump-outputs DIR`` writes what the headline's last timed step computed into ``DIR/<name>.npy`` (float32): its three
+losses and the weights after it, the item-indexed ones on a fixed sample of items (see ``dump_outputs``).  Inputs,
+initial weights and dropout draws are seeded, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -548,11 +554,57 @@ def w1_cold_row_frac(eng):
     return float(cold.float().mean().item())
 
 
+DUMP_SAMPLE_ITEMS = 32768
+
+
+def dump_outputs(ctx, eng, last_batch, out_dir):
+    """What the last timed step handed its caller: the step's losses (R, D, G) and the weights after it in the
+    reference's names and layouts, float32.  The item-indexed tensors (enc.lin1.weight columns, dec.lin3 rows) keep the
+    items of that step's batch plus a seeded draw of DUMP_SAMPLE_ITEMS items (all items when V is smaller): 800 bytes per
+    kept item, about 30 MB at the MPD shape; each rank cuts its own item range on the device.  Reading W1 needs its
+    pending zero-gradient Adam steps applied (flush_w1); the engine's state is restored afterwards, so the legs that
+    follow start from the state the timed steps left.  Collective over the item shards; rank 0 writes."""
+    import torch
+    from aaerec_b200.engine import enc_block_sizes, dec_block_sizes, disc_block_sizes
+    items = np.union1d(last_batch[1], np.random.RandomState(0).choice(eng.V, min(eng.V, DUMP_SAMPLE_ITEMS), replace=False))
+    snap, w1_dirty = eng._snapshot(), eng._w1_dirty
+    eng.flush_w1()
+    loc = torch.as_tensor(items, dtype=torch.int64, device=eng.dev) - eng.v_begin
+    mine = (loc >= 0) & (loc < eng.Vloc)
+    loc = loc.clamp(0, max(eng.Vloc - 1, 0))
+
+    def sampled(t):
+        rows = torch.where(mine.view((-1,) + (1,) * (t.dim() - 1)), t[loc], torch.zeros((), device=eng.dev))
+        if eng.world > 1:                   # every sampled item lives on exactly one rank: the sum is that rank's row
+            import torch.distributed as dist
+            dist.all_reduce(rows, group=eng.group)
+        return rows.cpu().numpy()
+    out = {"losses": eng.losses.cpu().numpy(), "enc.lin1.weight": sampled(eng.W1t).T,
+           "dec.lin3.weight": sampled(eng.Wd3), "dec.lin3.bias": sampled(eng.bd3)}
+    H, Cc = eng.H, eng.C
+    shapes = {"enc.lin2.weight": (H, H), "enc.lin3.weight": (Cc, H), "dec.lin1.weight": (H, eng.Cp),
+              "dec.lin2.weight": (H, H), "disc.lin1.weight": (H, Cc), "disc.lin2.weight": (H, H), "disc.lin3.weight": (1, H)}
+    for blk, sizes in ((eng.enc, enc_block_sizes(H, Cc)), (eng.dec, dec_block_sizes(H, eng.Cp)),
+                       (eng.disc, disc_block_sizes(H, Cc))):
+        off = 0
+        for name, sz in sizes:
+            out[name] = blk[off:off + sz].cpu().numpy().reshape(shapes.get(name, (sz,)))
+            off += sz
+    eng._restore(snap)
+    eng._w1_dirty = w1_dirty
+    del snap
+    if ctx.rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def train_workload(ctx, name, K, W, with_roofline=True, with_sustained=True, B=None, cond_dim=0, with_e2e=True,
-                   hot_w1=False):
+                   hot_w1=False, dump_dir=None):
     """value / e2e / roofline of one training workload; returns (dict, engine, batches).  hot_w1: every W1 row starts
     with live Adam moments (as if every item had been in a recent batch): the worst case of the time-blocked sweep,
-    none of its rows is cold."""
+    none of its rows is cold.  dump_dir: write the outputs of the last timed step there (dump_outputs)."""
     import torch
     n_batches = min(K + W, 32 if WORKLOADS[name][0] > 500000 else 64)
     _, batches, V, B = make_batches(name, n_batches, cond_dim=cond_dim, B=B)
@@ -566,6 +618,8 @@ def train_workload(ctx, name, K, W, with_roofline=True, with_sustained=True, B=N
                    for ip, ii, cc in batches]
     from aaerec_b200 import _native as N
     sec = train_leg(ctx, eng, dev_batches, B, K, W)
+    if dump_dir is not None:
+        dump_outputs(ctx, eng, batches[(W + K - 1) % len(batches)], dump_dir)
     N.reset_launch_count()
     eng.set_batch_device(*dev_batches[0])
     launches = eng.launches_per_step() * K
@@ -740,7 +794,7 @@ def run_ours(args):
     sampler = ClockSampler(ctx.local) if rank == 0 else None
     if sampler:
         sampler.start()
-    main, eng, batches = train_workload(ctx, head, K, W)
+    main, eng, batches = train_workload(ctx, head, K, W, dump_dir=args.dump_outputs)
     clocks = sampler.stop() if sampler else None
     V, B = eng.V, WORKLOADS[head][5]
 
@@ -957,7 +1011,13 @@ def main():
     ap.add_argument("--skip-big", action="store_true", help="skip the B=10000 leg")
     ap.add_argument("--predict-batch", type=int, default=1000)
     ap.add_argument("--budget", type=float, default=120.0, help="reference arm: seconds of timed work before it stops")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the losses and (sampled) weights of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl in ("reference", "reference-predict"):
         run_reference(args, use_cuda=False)
     elif args.impl == "reference-gpu":

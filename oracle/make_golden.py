@@ -41,7 +41,7 @@ def _state(model):
 
 
 def run_case(ref, name, n, V, H, C, B, epochs, dropout, cond_dim=0, data_seed=0, mean_len=6,
-             store_weights=True, k=10, adversarial=True, model_kwargs=None, dae=False):
+             store_weights=True, store_init=True, k=10, adversarial=True, model_kwargs=None, dae=False):
     aae = ref.aae
     if dae:                     # aaerec/dae.py:144-314 (SURVEY 8(f)-3): the reference's DenoisingAutoEncoder
         import aaerec.dae
@@ -120,8 +120,9 @@ def run_case(ref, name, n, V, H, C, B, epochs, dropout, cond_dim=0, data_seed=0,
     if cond_dim:
         out["cond"] = cond
     if store_weights:
-        for k_, v in init.items():
-            out["init/" + k_] = v
+        if store_init:
+            for k_, v in init.items():
+                out["init/" + k_] = v
         for k_, v in final.items():
             out["final/" + k_] = v
     else:
@@ -271,6 +272,16 @@ def ranking_case(ref):
     print("ranking ok")
 
 
+def metrics_case(ref):
+    """The reference's (mean, std) of every metric on the seeded case of tests/test_ranking_metrics.py, for
+    test_oracle_metrics_match_reference where the reference package is absent."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_ranking_metrics import METRICS, reference_metrics
+    want = np.asarray(reference_metrics(ref), dtype=np.float64)
+    np.savez_compressed(os.path.join(GOLDEN, "metrics_reference.npz"), metrics=np.asarray(METRICS), want=want)
+    print("metrics_reference ok")
+
+
 def main():
     os.makedirs(GOLDEN, exist_ok=True)
     ref = load_reference()
@@ -284,7 +295,10 @@ def main():
     run_case(ref, "aae_small_dropout", n=130, V=257, H=24, C=10, B=50, epochs=2, dropout=(.2, .2))
     run_case(ref, "aae_small_nodrop", n=130, V=257, H=24, C=10, B=50, epochs=2, dropout=(0, 0))
     run_case(ref, "aae_small_cond", n=130, V=257, H=24, C=10, B=50, epochs=2, dropout=(.2, .2), cond_dim=7)
-    run_case(ref, "aae_h100_dropout", n=96, V=520, H=100, C=50, B=32, epochs=2, dropout=(.2, .2), mean_len=8)
+    # the H=100 cases keep no initial weights (no test reads them; init_params rebuilds them from the seed): each
+    # file stays under 1 MB
+    run_case(ref, "aae_h100_dropout", n=96, V=520, H=100, C=50, B=32, epochs=2, dropout=(.2, .2), mean_len=8,
+             store_init=False)
     # SURVEY 8(c) indicative configuration (losses + |W| sums only, weights rebuilt from the seed)
     run_case(ref, "aae_survey_nodrop", n=300, V=1000, H=100, C=50, B=100, epochs=1, dropout=(0, 0),
              mean_len=8, store_weights=False)
@@ -293,7 +307,7 @@ def main():
     # plain AutoEncoder (aae.py:221-458; AAERecommender(adversarial=False)): reconstruction phase only
     run_case(ref, "ae_small_dropout", n=130, V=257, H=24, C=10, B=50, epochs=2, dropout=(.2, .2), adversarial=False)
     run_case(ref, "ae_h100_cond", n=96, V=520, H=100, C=50, B=32, epochs=2, dropout=(.2, .2), mean_len=8, cond_dim=7,
-             adversarial=False)
+             adversarial=False, store_init=False)
     # non-default model options (pins the oracle only; the CUDA path is checked against the oracle in these modes by
     # tests/test_gpu_parity.py::test_edge_cases_empty_rows_unnormalized_prior_scale)
     run_case(ref, "aae_opts_unnorm_scale_lrs", n=130, V=257, H=24, C=10, B=50, epochs=2, dropout=(.2, .2),
@@ -302,7 +316,7 @@ def main():
     run_case(ref, "dae_small_dropout", n=130, V=257, H=24, C=10, B=50, epochs=2, dropout=(.2, .2), dae=True,
              model_kwargs=dict(noise_factor=0.3))
     run_case(ref, "dae_h100_cond", n=96, V=520, H=100, C=50, B=32, epochs=2, dropout=(.2, .2), mean_len=8, cond_dim=7,
-             dae=True)
+             dae=True, store_init=False)
     # sibling models on the same decoder output layer (SURVEY 8(f)-3)
     if "vae_small".startswith(only):
         run_vae_case(ref, "vae_small", n=130, V=257, H=24, C=10, B=50, epochs=2)
@@ -315,6 +329,8 @@ def main():
                          mean_len=8)
     if "ranking".startswith(only):
         ranking_case(ref)
+    if "metrics_reference".startswith(only):
+        metrics_case(ref)
 
 
 if __name__ == "__main__":

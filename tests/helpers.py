@@ -72,6 +72,35 @@ def oracle_replay(g, record_rng=False):
     return model, np.asarray(losses), rngs, batches
 
 
+def write_reference_standin(root):
+    """A stand-in for the reference's ``aaerec`` package under ``root``: every module and name the import block of
+    main.py:11-20 uses, as plain placeholders.  The overlay tests check which tree each name resolves to, which needs
+    the tree's layout, not its code.  Returns ``root`` (the directory that contains ``aaerec/``)."""
+    cls = "class %s(object):\n    pass\n"
+    modules = {
+        "__init__.py": "",
+        "base.py": cls % "Recommender",
+        "aae.py": "from .condition import ConditionList  # noqa: F401\nUSE_WANDB = True\n" + "".join(
+            cls % c for c in ("Encoder", "Decoder", "Discriminator", "AutoEncoder", "AdversarialAutoEncoder",
+                              "AAERecommender", "DecodingRecommender")),
+        "dae.py": "def zeros_noise(x, p):\n    return x\n" + "".join(
+            cls % c for c in ("DenoisingAutoEncoder", "DAERecommender")),
+        "vae.py": "".join(cls % c for c in ("VAE", "VAERecommender")),
+        "condition.py": "".join(cls % c for c in ("ConditionList", "PretrainedWordEmbeddingCondition",
+                                                   "CategoricalCondition")),
+        "datasets.py": cls % "Bags",
+        "evaluation.py": cls % "Evaluation",
+        "baselines.py": "".join(cls % c for c in ("RandomBaseline", "Countbased", "MostPopular")),
+        "svd.py": cls % "SVDRecommender",
+    }
+    pkg = os.path.join(str(root), "aaerec")
+    os.makedirs(pkg, exist_ok=True)
+    for name, src in modules.items():
+        with open(os.path.join(pkg, name), "w") as fh:
+            fh.write(src)
+    return str(root)
+
+
 def rel_err(a, b):
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)

@@ -103,42 +103,53 @@ def test_reference_evaluation_harness_runs_both_recommenders(tmp_path, monkeypat
         assert abs(mean - r_our[name]) <= 5e-3, (name, mean, r_our[name])
 
 
-def test_aaerec_overlay_package_resolves(monkeypatch):
+def test_aaerec_overlay_package_resolves(monkeypatch, tmp_path):
     """sys.path = [aae-recommender_b200, <reference>]: the recommender classes of aaerec.aae / aaerec.dae / aaerec.vae are
     ours, the rest of those modules' namespaces and every other aaerec module are the reference's (main.py:13-22 imports
-    keep working)."""
-    ref = _reference()
+    keep working).  The reference tree is a stand-in with the reference's module layout (helpers.write_reference_standin),
+    and the real reference too when its package is present."""
+    from helpers import write_reference_standin
     from oracle import reference_loader as RL
-    saved = {k: v for k, v in sys.modules.items() if k == "aaerec" or k.startswith("aaerec.")}
-    for k in saved:
-        del sys.modules[k]
+    trees = [write_reference_standin(tmp_path)]
+    if RL.reference_available():
+        RL.load_reference()              # gensim / docutils stubs for the real reference's imports
+        trees.append(RL.REFERENCE_ROOT)
     pkg = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "aae-recommender_b200")
-    monkeypatch.setenv("AAEREC_REFERENCE", RL.REFERENCE_ROOT)
-    monkeypatch.syspath_prepend(pkg)
-    try:
-        import aaerec
-        import aaerec.aae as A
-        from aaerec.condition import ConditionList, CategoricalCondition      # noqa: F401  (the reference's)
-        from aaerec.evaluation import Evaluation                              # noqa: F401
-        import aaerec_b200.aae as B
-        assert aaerec.REFERENCE_DIR is not None
-        assert A.AAERecommender is B.AAERecommender and A.AdversarialAutoEncoder is B.AdversarialAutoEncoder
-        # the recommenders of main.py:98-124 are the B200 classes, everything else of the module is the reference's
-        import aaerec.dae as Dm
-        import aaerec.vae as Vm
-        import aaerec_b200.decoding as BD
-        import aaerec_b200.dae as BDae
-        import aaerec_b200.vae as BVae
-        assert A.DecodingRecommender is BD.DecodingRecommender
-        assert Dm.DAERecommender is BDae.DAERecommender and Vm.VAERecommender is BVae.VAERecommender
-        assert A.reference_module is not None and A.Encoder is A.reference_module.Encoder
-        assert Dm.reference_module is not None and Dm.zeros_noise is Dm.reference_module.zeros_noise
-        assert Vm.reference_module is not None
-        assert ConditionList.__module__ == "aaerec.condition" and "aaerec_b200" not in ConditionList.__module__
-    finally:
-        for k in [k for k in sys.modules if k == "aaerec" or k.startswith("aaerec.")]:
+    for reference_root in trees:
+        saved = {k: v for k, v in sys.modules.items() if k == "aaerec" or k.startswith("aaerec.")}
+        for k in saved:
             del sys.modules[k]
-        sys.modules.update(saved)
+        try:
+            with monkeypatch.context() as m:
+                m.setenv("AAEREC_REFERENCE", reference_root)
+                m.syspath_prepend(pkg)
+                _check_overlay(reference_root)
+        finally:
+            for k in [k for k in sys.modules if k == "aaerec" or k.startswith("aaerec.")]:
+                del sys.modules[k]
+            sys.modules.update(saved)
+
+
+def _check_overlay(reference_root):
+    import aaerec
+    import aaerec.aae as A
+    from aaerec.condition import ConditionList, CategoricalCondition      # noqa: F401  (the reference's)
+    from aaerec.evaluation import Evaluation                              # noqa: F401
+    import aaerec_b200.aae as B
+    assert aaerec.REFERENCE_DIR == os.path.join(os.path.abspath(reference_root), "aaerec")
+    assert A.AAERecommender is B.AAERecommender and A.AdversarialAutoEncoder is B.AdversarialAutoEncoder
+    # the recommenders of main.py:98-124 are the B200 classes, everything else of the module is the reference's
+    import aaerec.dae as Dm
+    import aaerec.vae as Vm
+    import aaerec_b200.decoding as BD
+    import aaerec_b200.dae as BDae
+    import aaerec_b200.vae as BVae
+    assert A.DecodingRecommender is BD.DecodingRecommender
+    assert Dm.DAERecommender is BDae.DAERecommender and Vm.VAERecommender is BVae.VAERecommender
+    assert A.reference_module is not None and A.Encoder is A.reference_module.Encoder
+    assert Dm.reference_module is not None and Dm.zeros_noise is Dm.reference_module.zeros_noise
+    assert Vm.reference_module is not None
+    assert ConditionList.__module__ == "aaerec.condition" and "aaerec_b200" not in ConditionList.__module__
 
 
 def test_phase_methods_equal_partial_fit():
