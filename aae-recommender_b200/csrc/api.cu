@@ -1,7 +1,7 @@
 // C-ABI glue: error reporting, device check and the dispatchers of the decoder output layer.
 #include <stdarg.h>
 #include <string.h>
-#include "common.cuh"
+#include "dec_out.cuh"
 
 namespace aae {
 
@@ -37,24 +37,6 @@ int sm_count() {
   }
   return n;
 }
-
-int dec_out_train_simt(const float* h2, int B, int H, float* Wd3, float* bd3, float* mW, float* vW, float* mb,
-                       float* vb, int v_begin, int Vloc, const int32_t* indptr, const int32_t* indices, double n_total,
-                       const aae_step_state* st, float* dh2, double* loss_sum, cudaStream_t s);
-int dec_out_scores_simt(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int apply_sigmoid,
-                        float* out, int64_t ldo, cudaStream_t s);
-int dec_out_train_tc(const float* h2, int B, int H, float* Wd3, float* bd3, float* mW, float* vW, float* mb, float* vb,
-                     int v_begin, int Vloc, const int32_t* indptr, const int32_t* indices, double n_total,
-                     const aae_step_state* st, float* dh2, double* loss_sum, int split, bool pipelined, float* gwork,
-                     cudaStream_t s);
-int tc2_max_rows(int H);
-int dec_out_scores_tc(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int apply_sigmoid,
-                      float* out, int64_t ldo, int split, cudaStream_t s);
-
-void trace_set_bag(unsigned long long* p);
-void trace_set_mlp(unsigned long long* p);
-void trace_set_tc(unsigned long long* p);
-void trace_set_w1b(unsigned long long* p);
 
 }  // namespace aae
 
@@ -134,10 +116,8 @@ int aae_dec_out_scores(const float* h2, int B, int H, const float* Wd3, const fl
   AAE_REQUIRE(h2 && Wd3 && bd3 && out, "null pointer");
   AAE_REQUIRE(B > 0 && H > 0 && Vloc > 0 && ldo >= Vloc, "bad size");
   if (impl == 0) return dec_out_scores_simt(h2, B, H, Wd3, bd3, Vloc, apply_sigmoid, out, ldo, as_stream(stream));
-  if (impl == 1 || impl == 2)
-    return dec_out_scores_tc(h2, B, H, Wd3, bd3, Vloc, apply_sigmoid, out, ldo, impl == 1 ? 3 : 1, as_stream(stream));
-  if (impl == 3 || impl == 4)   // the first-cut, unpipelined tensor-core kernel (A/B reference)
-    return dec_out_scores_tc(h2, B, H, Wd3, bd3, Vloc, apply_sigmoid, out, ldo, impl == 3 ? 13 : 11, as_stream(stream));
+  if (impl >= 1 && impl <= 4)   // 3/4 score as 1/2: the training-only choice of kernel has no counterpart here
+    return dec_out_scores_tc(h2, B, H, Wd3, bd3, Vloc, apply_sigmoid, out, ldo, (impl & 1) ? 3 : 1, as_stream(stream));
   set_error("dec_out_scores: unknown impl %d", impl);
   return AAE_E_ARG;
 }

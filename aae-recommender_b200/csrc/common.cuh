@@ -122,6 +122,10 @@ __device__ __forceinline__ void trace_mark(int id, int end) {
 }
 #define AAE_DEFINE_TRACE_SETTER(name)                                                    \
   void name(unsigned long long* p) { cudaMemcpyToSymbol(g_trace_buf, &p, sizeof(p)); }
+void trace_set_bag(unsigned long long* p);   // bag.cu
+void trace_set_mlp(unsigned long long* p);   // mlp.cu
+void trace_set_tc(unsigned long long* p);    // dec_out_tc.cu
+void trace_set_w1b(unsigned long long* p);   // w1_blocked.cu
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -1,6 +1,6 @@
 // K5 v2: predict's candidate filter fed by TMA, W' tiles multicast across a thread-block cluster.
 //
-// The first K5 (dec_out_tc.cu, dec_out_select_kernel) ran every logit through the fp32-accurate 3xTF32 split and fed
+// The first K5 (dec_out_select.cu, dec_out_select_kernel) ran every logit through the fp32-accurate 3xTF32 split and fed
 // the tensor core from register-staged loads: each of the row-chunk CTAs that walk the same W' tile fetched it from
 // L2 and converted it to operand layout by itself, and the kernel was bound by that loader, not by the MMAs
 // (single-pass TF32 was no faster).  An exact top-k does not need exact logits for all B x V pairs -- only for the
@@ -29,7 +29,8 @@
 #include <map>
 #include <mutex>
 #include <tuple>
-#include "common.cuh"
+#include "tcgen05.cuh"
+#include "dec_out.cuh"
 
 namespace aae {
 namespace s2 {
@@ -49,115 +50,6 @@ constexpr int NWE = 16;                 // epilogue warps
 constexpr int NT = 32 * (NWE + 2);      // + MMA warp + TMA warp
 constexpr int CW = PN / 4;              // accumulator columns per epilogue thread
 constexpr uint32_t T_ACC = 0, T_A = 256, TMEM_COLS = 512;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (!done) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, 0x989680;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}\n"
-        : "=r"(done)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (!done && ++spins > (1u << 24)) __trap();      // a lost completion must not hang the device
-  }
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}\n" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ float tf32_hi(float x) { return __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
-
-// one box of a W' tile, multicast to every CTA of the cluster named in `mask` (same stage offset, same barrier offset)
-__device__ __forceinline__ void tma_load_mc(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, %3}], "
-      "[%4], %5;" ::"r"(smem_u32(dst)),
-      "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar)), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(
-          smem_u32(dst)),
-      "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar))
-      : "memory");
-}
-// K-major operand, SWIZZLE_32B (layout type 6): rows of 32 bytes, SBO = 256 bytes between 8-row groups
-__device__ __forceinline__ uint64_t make_desc_sw32(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFFu);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(256u >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)6 << 61;
-  return d;
-}
-// K-major operand, SWIZZLE_128B (layout type 2), SBO = 1024 bytes between 8-row groups, Blackwell descriptor version
-__device__ __forceinline__ uint64_t make_desc_sw128(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFFu);
-  d |= (uint64_t)1 << 16;                       // LBO (unused for swizzled K-major layouts)
-  d |= (uint64_t)(1024u >> 4) << 32;            // SBO
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);   // tf32 x tf32 -> f32
-}
-__device__ __forceinline__ void mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}\n" ::"r"(d_tmem),
-      "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void mma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld16_issue(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait32(uint32_t* r) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
-                 "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]),
-                 "+r"(r[16]), "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]),
-                 "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])::"memory");
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const float* v) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr),
-               "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])),
-               "r"(__float_as_uint(v[3])), "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])),
-               "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7]))
-               : "memory");
-}
 
 struct Sel2Args {
   const float* h2; int B, H;
@@ -189,11 +81,7 @@ __global__ void __launch_bounds__(NT, 1) dec_out_select2_kernel(const __grid_con
   // against 0.88 us when the clusters read different tiles); HBM has the bandwidth to stream W' once per cluster row.
   const int rot = (groups_per_pass > 1 && n_my > 0) ? (int)(((long long)((int)blockIdx.y / CY) * n_my) / groups_per_pass) : 0;
 
-  if (warp == NWE) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == NWE) tmem_alloc(&tmem_base_s, TMEM_COLS);
   if (tid == 0) {
     for (int s = 0; s < NSTAGE; ++s) {
       mbar_init(&bar_full[s], 1);
@@ -237,7 +125,7 @@ __global__ void __launch_bounds__(NT, 1) dec_out_select2_kernel(const __grid_con
         }
         tmem_st8(lane_addr + T_A + c * 8, hi);
       }
-      asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+      tmem_st_wait();
     }
     tc_fence_before();
     __syncthreads();
@@ -249,7 +137,7 @@ __global__ void __launch_bounds__(NT, 1) dec_out_select2_kernel(const __grid_con
         for (int i = 0; i < n_my; ++i, ++it_p) {
           const int s = (int)(it_p % NSTAGE);
           const uint32_t use = it_p / NSTAGE;
-          mbar_wait(&bar_empty[s], (use & 1u) ^ 1u);          // every CTA of the cluster has released the stage
+          mbar_wait_spin(&bar_empty[s], (use & 1u) ^ 1u);          // every CTA of the cluster has released the stage
           mbar_arrive_expect_tx(&bar_full[s], STAGE_BYTES);   // the whole tile lands here (all slices, all senders)
           int j = i + rot;
           if (j >= n_my) j -= n_my;
@@ -270,8 +158,8 @@ __global__ void __launch_bounds__(NT, 1) dec_out_select2_kernel(const __grid_con
       // ================= MMA issuer =================
       for (int i = 0; i < n_my; ++i, ++it_m) {
         const int s = (int)(it_m % NSTAGE), acc = (int)(it_m & 1u);
-        mbar_wait(&bar_full[s], (it_m / NSTAGE) & 1u);
-        mbar_wait(&bar_acc_empty[acc], ((it_m >> 1) & 1u) ^ 1u);
+        mbar_wait_spin(&bar_full[s], (it_m / NSTAGE) & 1u);
+        mbar_wait_spin(&bar_acc_empty[acc], ((it_m >> 1) & 1u) ^ 1u);
         tc_fence_after();
         if (elect_one()) {
           const uint32_t sbase = smem_u32(stages + (size_t)s * STAGE_BYTES);
@@ -305,11 +193,11 @@ __global__ void __launch_bounds__(NT, 1) dec_out_select2_kernel(const __grid_con
         int jt = i + rot;
         if (jt >= n_my) jt -= n_my;
         const int v0 = ((int)blockIdx.x + jt * (int)gridDim.x) * a.tile_stride * PN;
-        mbar_wait(&bar_acc_full[acc], (it_e >> 1) & 1u);
+        mbar_wait_spin(&bar_acc_full[acc], (it_e >> 1) & 1u);
         tc_fence_after();
         uint32_t zr[CW];
-        tmem_ld16_issue(lane_addr + T_ACC + (uint32_t)(acc * PN + c0), zr);
-        tmem_ld16_issue(lane_addr + T_ACC + (uint32_t)(acc * PN + c0 + 16), zr + 16);
+        TmemIO<16>::ld_issue(lane_addr + T_ACC + (uint32_t)(acc * PN + c0), zr);
+        TmemIO<16>::ld_issue(lane_addr + T_ACC + (uint32_t)(acc * PN + c0 + 16), zr + 16);
         tmem_ld_wait32(zr);
         tc_fence_before();
         __syncwarp();
@@ -350,7 +238,7 @@ __global__ void __launch_bounds__(NT, 1) dec_out_select2_kernel(const __grid_con
   tc_fence_before();
   __syncthreads();
   if (CY > 1) cg::this_cluster().sync();         // no CTA leaves while a peer may still multicast into its stages
-  if (warp == NWE) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS) : "memory");
+  if (warp == NWE) tmem_dealloc(tmem, TMEM_COLS);
 }
 
 // W' = [Wd3 | bd3 | 0 0 0] as a padded [Vloc, KP] matrix + the largest row norm (for the TF32 error bound)

@@ -2,9 +2,9 @@
 // Training: logits, sigmoid, BCE, dZ, dh2 += dZ.W, dW = dZ^T.h2 and Adam on W/bias in ONE pass over
 // Wd3 (the [B,V] logit matrix never exists in HBM).  Prediction: scores (logits or probabilities).
 // This is the exact-fp32 correctness baseline and the path for shapes outside the tensor-core
-// kernel's envelope; the tcgen05 kernel in dec_out_tc.cu is the fast path.
+// kernels' envelope; the tcgen05 kernels in dec_out_tc.cu (training) and dec_out_select.cu (scores) are the fast path.
 // Reference: aaerec/aae.py:176-177 (lin3 + sigmoid), :693-695 (BCE), :703 (backward), :707 (dec_optim).
-#include "common.cuh"
+#include "dec_out.cuh"
 
 namespace aae {
 

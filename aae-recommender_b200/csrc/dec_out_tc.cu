@@ -1,5 +1,7 @@
-// K3/K5 tensor-core variant: the n_items-wide decoder output layer on tcgen05 (5th-gen tensor
-// cores, accumulators in TMEM), fp32-accurate through a 3xTF32 split.
+// K3: the n_items-wide decoder output layer, training, on tcgen05 (5th-gen tensor cores, accumulators in
+// TMEM), fp32-accurate through a 3xTF32 split.  Two kernels (one tile at a time; the role-split pipeline
+// that is the default for the reference's shapes), their launchers and the operand self-test.  The PTX
+// wrappers and the K-major hi/lo operand layer are in tcgen05.cuh.
 //
 // Per tile of TN=32 items and a batch of up to 128 rows, three GEMMs (each operand kept as a tf32
 // "hi" part and an fp32 remainder "lo"; x = hi + lo exactly; products issued as hi*hi + lo*hi + hi*lo,
@@ -20,14 +22,9 @@
 // and applies Adam in registers.  Logits never reach HBM.
 //
 // Reference: aaerec/aae.py:176-177 (lin3 + sigmoid), :693-695 (BCE), :703 (backward), :707 (dec_optim).
-#include "common.cuh"
+#include "tcgen05.cuh"
+#include "dec_out.cuh"
 
-#ifndef TC_WAIT_HINT
-#define TC_WAIT_HINT 0x989680u
-#endif
-#ifndef TC_WAIT_SLEEP_NS
-#define TC_WAIT_SLEEP_NS 40
-#endif
 #ifndef TC2_CW
 #define TC2_CW 16   // accumulator columns per epilogue thread of the pipelined kernel (two roles of 8 warps each)
 #endif
@@ -39,189 +36,9 @@ namespace aae {
 AAE_DEFINE_TRACE_SETTER(trace_set_tc)
 namespace tc {
 
-constexpr int TN = 32;          // items per tile
-constexpr int BM = 128;         // batch rows per chunk (MMA M)
 constexpr int NT = 512;         // threads: 16 warps = 4 TMEM lane quarters x 4 column parts
 constexpr int CW = 8;           // accumulator columns per thread in the epilogues
-constexpr int CORE = 128;       // bytes of one core matrix (8 rows x 16 B)
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// shared-memory matrix descriptor, SWIZZLE_NONE, Blackwell version bit
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFFu);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32;
-  d |= (uint64_t)1 << 46;
-  return d;
-}
-// the same with a swizzle mode in bits [61,64) (1 = SWIZZLE_128B_BASE32B: the layout of MN-major 32-bit operands)
-__device__ __forceinline__ uint64_t make_desc_sw(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout_type) {
-  return make_desc(saddr, lbo_bytes, sbo_bytes) | ((uint64_t)layout_type << 61);
-}
-// instruction descriptor for kind::tf32, fp32 accumulate
-__host__ __device__ constexpr uint32_t make_idesc(int M, int N, int a_mn_major, int b_mn_major) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
-         ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void mma_tf32(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                         uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-      "}\n" ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// A operand from TMEM (lanes = M, columns = K), B from shared memory
-__device__ __forceinline__ void mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t"
-      "}\n" ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t done = 0;
-  uint32_t spins = 0;
-  while (!done) {
-    if (spins) __nanosleep(TC_WAIT_SLEEP_NS);   // back off: spinning warps steal issue slots from the MMA issuer
-    if (++spins > (1u << 22)) __trap();          // a lost MMA completion must not hang the device
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}\n"
-        : "=r"(done)
-        : "r"(smem_u32(bar)), "r"(parity), "r"(TC_WAIT_HINT)   // suspend-time hint: sleep in hardware, do not spin
-        : "memory");
-  }
-}
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "elect.sync _|p, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t"
-      "}\n"
-      : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-__device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)),
-               "r"(ncols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// 16 consecutive fp32 columns of this thread's TMEM lane
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float* v) {
-  uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// store 16 consecutive fp32 columns of this thread's TMEM lane
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const float* v) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
-      "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])),
-      "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7])),
-      "r"(__float_as_uint(v[8])), "r"(__float_as_uint(v[9])), "r"(__float_as_uint(v[10])), "r"(__float_as_uint(v[11])),
-      "r"(__float_as_uint(v[12])), "r"(__float_as_uint(v[13])), "r"(__float_as_uint(v[14])), "r"(__float_as_uint(v[15]))
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float* v) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-// issue only: the registers are valid after tmem_ld8_wait (which ties them to the wait)
-__device__ __forceinline__ void tmem_ld8_issue(uint32_t taddr, uint32_t* r) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld8_wait(uint32_t* r, float* v) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7])::"memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const float* v) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr),
-               "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])),
-               "r"(__float_as_uint(v[3])), "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])),
-               "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7]))
-               : "memory");
-}
-// N-column variants used by the pipelined kernel (N = 8 or 16)
-template <int N> struct TmemIO;
-template <> struct TmemIO<8> {
-  static __device__ __forceinline__ void ld_issue(uint32_t taddr, uint32_t* r) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                 : "r"(taddr)
-                 : "memory");
-  }
-  static __device__ __forceinline__ void ld_wait(uint32_t* r) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7])::"memory");
-  }
-  static __device__ __forceinline__ void st(uint32_t taddr, const float* v) { tmem_st8(taddr, v); }
-};
-template <> struct TmemIO<16> {
-  static __device__ __forceinline__ void ld_issue(uint32_t taddr, uint32_t* r) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr)
-        : "memory");
-  }
-  static __device__ __forceinline__ void ld_wait(uint32_t* r) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
-                   "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])::"memory");
-  }
-  static __device__ __forceinline__ void st(uint32_t taddr, const float* v) { tmem_st16(taddr, v); }
-};
-__device__ __forceinline__ float tf32_hi(float x) { return __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
 // Pins a prefetched register tile to its point of use: without it the compiler hoists the hi/lo split (pure ALU work
 // on the loaded values) up to right behind the global loads, and the warp then waits for the load latency one
 // iteration early, in the middle of the pipeline, instead of letting it overlap the MMAs of that iteration.
@@ -232,100 +49,6 @@ __device__ __forceinline__ void pin4(float4& x) {
 #if TC_PIN_PREFETCH
   asm volatile("" : "+f"(x.x), "+f"(x.y), "+f"(x.z), "+f"(x.w));
 #endif
-}
-
-// byte offset of element (r, c) in a core-matrix-tiled buffer whose row groups are `s_r` bytes apart
-__device__ __forceinline__ uint32_t core_off(int r, int c, uint32_t s_r) {
-  return (uint32_t)(r >> 3) * s_r + (uint32_t)(c >> 2) * CORE + (uint32_t)(r & 7) * 16u + (uint32_t)(c & 3) * 4u;
-}
-// store 4 consecutive columns (one 16-byte chunk) of row r as hi / lo
-__device__ __forceinline__ void store_split4(unsigned char* hi, unsigned char* lo, int r, int cg, uint32_t s_r,
-                                             float4 x, bool with_lo) {
-  uint32_t off = (uint32_t)(r >> 3) * s_r + (uint32_t)cg * CORE + (uint32_t)(r & 7) * 16u;
-  float4 h = make_float4(tf32_hi(x.x), tf32_hi(x.y), tf32_hi(x.z), tf32_hi(x.w));
-  *reinterpret_cast<float4*>(hi + off) = h;
-  if (with_lo) *reinterpret_cast<float4*>(lo + off) = make_float4(x.x - h.x, x.y - h.y, x.z - h.z, x.w - h.w);
-}
-
-// Descriptors of one operand (hi and lo parts) with the per-k-step increment of the start-address
-// field (units of 16 bytes); built once per kernel.
-struct SmemOp {
-  uint64_t hi, lo;
-  uint32_t step16;
-};
-__device__ __forceinline__ SmemOp make_op(const void* hi, const void* lo, uint32_t lbo, uint32_t sbo, uint32_t step) {
-  SmemOp o;
-  o.hi = make_desc(smem_u32(hi), lbo, sbo);
-  o.lo = make_desc(smem_u32(lo), lbo, sbo);
-  o.step16 = step >> 4;
-  return o;
-}
-// One GEMM, both operands in shared memory: up to 16 k-steps x (1 or 3) tcgen05.mma.  Fully unrolled with a
-// warp-uniform bound so that the descriptor arithmetic stays on constants (the issuing lane executes a few
-// instructions per MMA instead of rebuilding descriptors).
-template <int SPLIT>
-__device__ __forceinline__ void issue_gemm(uint32_t d_tmem, const SmemOp& a, const SmemOp& b, int ksteps,
-                                           uint32_t idesc, uint32_t first_acc) {
-#pragma unroll
-  for (int k = 0; k < 16; ++k) {
-    if (k < ksteps) {
-      const uint32_t acc = (k == 0) ? first_acc : 1u;
-      const uint64_t ah = a.hi + (uint64_t)(k * a.step16), bh = b.hi + (uint64_t)(k * b.step16);
-      if (SPLIT == 3) {
-        mma_tf32(d_tmem, a.lo + (uint64_t)(k * a.step16), bh, idesc, acc);
-        mma_tf32(d_tmem, ah, b.lo + (uint64_t)(k * b.step16), idesc, 1u);
-        mma_tf32(d_tmem, ah, bh, idesc, 1u);
-      } else {
-        mma_tf32(d_tmem, ah, bh, idesc, acc);
-      }
-    }
-  }
-}
-// One GEMM with the A operand in TMEM: k-step s reads A columns [8s, 8s+8).
-template <int SPLIT>
-__device__ __forceinline__ void issue_gemm_ts(uint32_t d_tmem, uint32_t a_hi_t, uint32_t a_lo_t, const SmemOp& b,
-                                              int ksteps, uint32_t idesc, uint32_t first_acc) {
-#pragma unroll
-  for (int k = 0; k < 16; ++k) {
-    if (k < ksteps) {
-      const uint32_t acc = (k == 0) ? first_acc : 1u;
-      const uint64_t bh = b.hi + (uint64_t)(k * b.step16);
-      if (SPLIT == 3) {
-        mma_tf32_ts(d_tmem, a_lo_t + 8 * k, bh, idesc, acc);
-        mma_tf32_ts(d_tmem, a_hi_t + 8 * k, b.lo + (uint64_t)(k * b.step16), idesc, 1u);
-        mma_tf32_ts(d_tmem, a_hi_t + 8 * k, bh, idesc, 1u);
-      } else {
-        mma_tf32_ts(d_tmem, a_hi_t + 8 * k, bh, idesc, acc);
-      }
-    }
-  }
-}
-
-// Shared-memory operand geometry (all K-major, no swizzle; LBO = stride between 16-byte column
-// groups along K, SBO = stride between 8-row groups along M/N).
-struct Geom {
-  int H, Kp, Np;             // hidden, K of G1 padded to 8 (H+1 -> Kp), N of G2 padded to 16
-  uint32_t hb_sbo, wb_sbo;   // Hb [128][Kp], Wb [32][Kp]: LBO = CORE
-  uint32_t wt_lbo, wt_sbo;   // Wtb [Np][32]  (rows = hidden unit, cols = item)
-  uint32_t dt_lbo, dt_sbo;   // Dtb [32][128] (rows = item, cols = batch row)
-  uint32_t hb_bytes, wb_bytes, wt_bytes, dt_bytes;
-};
-__host__ __device__ inline Geom make_geom(int H) {
-  Geom g;
-  g.H = H;
-  g.Kp = (H + 1 + 7) & ~7;
-  g.Np = (g.Kp + 15) & ~15;
-  g.hb_sbo = (uint32_t)(g.Kp / 4) * CORE;
-  g.wb_sbo = (uint32_t)(g.Kp / 4) * CORE;
-  g.wt_lbo = CORE + 16;                     // +16: the transposing stores of the W' tile are conflict-free
-  g.wt_sbo = (TN / 4) * g.wt_lbo;
-  g.dt_lbo = CORE + 16;                     // +16: the E1 transposing stores become conflict-free
-  g.dt_sbo = (BM / 4) * g.dt_lbo;
-  g.hb_bytes = (BM / 8) * g.hb_sbo;
-  g.wb_bytes = (TN / 8) * g.wb_sbo;
-  g.wt_bytes = (uint32_t)(g.Np / 8) * g.wt_sbo;
-  g.dt_bytes = (TN / 8) * g.dt_sbo;
-  return g;
 }
 __host__ __device__ inline size_t smem_bytes(const Geom& g) {
   return 2 * ((size_t)g.hb_bytes + g.wb_bytes + g.wt_bytes + g.dt_bytes) + 256;
@@ -564,7 +287,7 @@ __global__ void __launch_bounds__(NT, 1) dec_out_train_tc_kernel(
         }
       }
     }
-    mbar_wait(&bar_mma, phase);
+    mbar_wait_backoff(&bar_mma, phase);
     phase ^= 1;
     tc_fence_after();
     // ---- E1: sigmoid + BCE + dZ for (row brow, columns 8*cpart .. +7)
@@ -600,7 +323,7 @@ __global__ void __launch_bounds__(NT, 1) dec_out_train_tc_kernel(
       __syncwarp();
     }
     dh_started = true;
-    mbar_wait(&bar_mma, phase);
+    mbar_wait_backoff(&bar_mma, phase);
     phase ^= 1;
     tc_fence_after();
     // ---- E2: Adam on (hidden unit k, items 8*cpart .. +7): coalesced over k
@@ -652,42 +375,6 @@ __global__ void __launch_bounds__(NT, 1) dec_out_train_tc_kernel(
   if (warp == 0) tmem_dealloc(tmem, TMEM_COLS);
 }
 
-// Row cursor with three entries of lookahead: n0 = indices[pos] is compared every tile; n1..n3 were requested
-// when the cursor last moved, so a compare only waits on a load when the row has four items within one
-// stretch of tiles (the stall would otherwise hit every warp: 32 rows advance independently).
-struct RowCursor2 {
-  int pos, end, n0, n1, n2, n3;
-};
-__device__ __forceinline__ void cursor_init(RowCursor2& c, const int32_t* __restrict__ indices, int pos, int end) {
-  c.pos = pos;
-  c.end = end;
-  c.n0 = (pos < end) ? __ldg(indices + pos) : 0x7fffffff;
-  c.n1 = (pos + 1 < end) ? __ldg(indices + pos + 1) : 0x7fffffff;
-  c.n2 = (pos + 2 < end) ? __ldg(indices + pos + 2) : 0x7fffffff;
-  c.n3 = (pos + 3 < end) ? __ldg(indices + pos + 3) : 0x7fffffff;
-}
-__device__ __forceinline__ void cursor_advance(RowCursor2& c, const int32_t* __restrict__ indices) {
-  c.n0 = c.n1;
-  c.n1 = c.n2;
-  c.n2 = c.n3;
-  ++c.pos;
-  c.n3 = (c.pos + 3 < c.end) ? __ldg(indices + c.pos + 3) : 0x7fffffff;
-}
-// bits of the items of [v0g, v0g + TN) in the row; first skips the row's items below v0g
-__device__ __forceinline__ uint32_t tile_targets2(RowCursor2& c, const int32_t* __restrict__ indices, int v0g) {
-  while (c.n0 < v0g) cursor_advance(c, indices);
-  uint32_t m = 0;
-  while (c.n0 < v0g + TN) {
-    m |= 1u << (c.n0 - v0g);
-    cursor_advance(c, indices);
-  }
-  return m;
-}
-__device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes) {
-  if (bytes >= 16u)
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes & ~15u) : "memory");
-}
-
 // ---------------------------------------------------------------------------------------------
 // Pipelined training kernel (the default for the reference's shapes).  Same three GEMMs and epilogues as
 // above, as a role-split pipeline of 18 warps (CWT = 16 accumulator columns per epilogue thread):
@@ -713,8 +400,10 @@ constexpr uint32_t T2_Z = 0, T2_DW = 64, T2_DZH = 128, T2_DZL = 160, T2_DH = 192
 __device__ __forceinline__ void named_bar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 __device__ __forceinline__ void named_bar_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 
-// target 0 and |z| < 16: ATen's clamped formula (common.cuh bce_term) equals softplus(z) / sigmoid(z)/N to
-// far below 1e-6 relative; everything else goes through bce_term.
+// MUFU approximations of the BCE fast paths (target 0 and |z| < 16, where ATen's clamped formula, common.cuh bce_term,
+// equals softplus(z) / sigmoid(z)/N to far below 1e-6 relative; everything else goes through bce_term).  log(1+u)
+// through lg2 has an absolute error of one rounding of 1+u (6e-8, unbiased) per element: invisible in the mean over
+// B*V terms; the gradient sigmoid(z)/N is accurate to ~2 ulp.
 __device__ __forceinline__ float ex2_approx(float x) {
   float r;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
@@ -724,17 +413,6 @@ __device__ __forceinline__ float lg2_approx(float x) {
   float r;
   asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
   return r;
-}
-// ~15 instructions: u = e^-|z| (one ex2), 1/(1+u) (one rcp), log(1+u) (one lg2).  log(1+u) through lg2 has an
-// absolute error of one rounding of 1+u (6e-8, unbiased) per element: invisible in the mean over B*V terms;
-// the gradient sigmoid(z)/N is accurate to ~2 ulp.
-__device__ __forceinline__ float bce_neg_fast(float z, float inv_n, float& dz) {
-  float u = ex2_approx(-1.4426950408889634f * fabsf(z));
-  float t = 1.0f + u;
-  float r = rcp_approx(t);
-  float x = (z >= 0.f) ? r : u * r;
-  dz = x * inv_n;
-  return fmaf(lg2_approx(t), 0.6931471805599453f, fmaxf(z, 0.f));
 }
 
 // this thread's share of the W' tile when NW warps split the Kp/4 (<= 32) 16-byte column groups
@@ -797,20 +475,6 @@ __device__ __forceinline__ void store_wt_regs(const float4* wr, const WChunk* wc
       tl[0] = x.x - h.x; tl[4] = x.y - h.y; tl[8] = x.z - h.z; tl[12] = x.w - h.w;
     }
   }
-}
-
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// TMA bulk copy global -> shared (contiguous bytes, 16-byte aligned), completion counted on an mbarrier
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_u32(dst_smem)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
 }
 
 #ifndef K3_PF_MV
@@ -1016,7 +680,7 @@ __global__ void __launch_bounds__(Tc2Cfg<CWT>::NTHR, 1) dec_out_train_tc2_kernel
         K3X_MARK(it, 14);
       }
       if (it > 2) {                 // G3(it-1) overwrites the dW'^T buffer that E2(it-3) reads
-        if ((it - 1) & 1) { mbar_wait(&bar_dwfree[1], ph_f1); ph_f1 ^= 1; } else { mbar_wait(&bar_dwfree[0], ph_f0); ph_f0 ^= 1; }
+        if ((it - 1) & 1) { mbar_wait_backoff(&bar_dwfree[1], ph_f1); ph_f1 ^= 1; } else { mbar_wait_backoff(&bar_dwfree[0], ph_f0); ph_f0 ^= 1; }
         tc_fence_after();
       }
       if (elect_one()) {
@@ -1179,7 +843,7 @@ __global__ void __launch_bounds__(Tc2Cfg<CWT>::NTHR, 1) dec_out_train_tc2_kernel
 
       // ---- E1(i), math part: needs only G1(i)
       if (warp == 0) K3X_MARK(i, 2);
-      mbar_wait(&bar_g1, phase);
+      mbar_wait_backoff(&bar_g1, phase);
       tc_fence_after();
       if (warp == 0) K3X_MARK(i, 3);
       float dzh[CWT], dzl[CWT];
@@ -1306,7 +970,7 @@ __global__ void __launch_bounds__(Tc2Cfg<CWT>::NTHR, 1) dec_out_train_tc2_kernel
       }
       // ---- operand stores: need G2/G3(i-1) to be done with dZ, Dtb and Wtb
       if (warp == 0) K3X_MARK(i, 4);
-      mbar_wait(&bar_g23, phase);
+      mbar_wait_backoff(&bar_g23, phase);
       phase ^= 1;
       tc_fence_after();
       if (warp == 0) K3X_MARK(i, 5);
@@ -1333,7 +997,7 @@ __global__ void __launch_bounds__(Tc2Cfg<CWT>::NTHR, 1) dec_out_train_tc2_kernel
         load_w_regs_t<WCHT>(wB, wc, Wd3, bd3, H, t2 * TN, min(TN, Vloc - t2 * TN));
       }
     }
-    mbar_wait(&bar_g23, phase);                       // G2/G3 of the last tile
+    mbar_wait_backoff(&bar_g23, phase);                       // G2/G3 of the last tile
     tc_fence_after();
     if (warp == 0) K3X_MARK(39, 6);
     // ---- flush dh2 (lane = batch row, columns = hidden unit) while the E2 warps finish the last tile; the column
@@ -1416,7 +1080,7 @@ __global__ void __launch_bounds__(Tc2Cfg<CWT>::NTHR, 1) dec_out_train_tc2_kernel
       }
       // old W/m/v from the TMA-filled stage; the stage is handed back for the refill as soon as it has been read
       if (warp == NWE) K3X_MARK(jt, 8);
-      mbar_wait(&bar_stage, phase_e);
+      mbar_wait_backoff(&bar_stage, phase_e);
       phase_e ^= 1;
       if (warp == NWE) K3X_MARK(jt, 9);
 #ifdef K3X_NO_E2LD
@@ -1454,7 +1118,7 @@ __global__ void __launch_bounds__(Tc2Cfg<CWT>::NTHR, 1) dec_out_train_tc2_kernel
         named_bar_arrive(2 + (int)(dep & rt_zero), NTT);
       }
       // dW'^T(jt): its own mbarrier per TMEM buffer (these warps run behind the MMA warp by up to two tiles)
-      if (jt & 1) { mbar_wait(&bar_dw[1], ph_dw1); ph_dw1 ^= 1; } else { mbar_wait(&bar_dw[0], ph_dw0); ph_dw0 ^= 1; }
+      if (jt & 1) { mbar_wait_backoff(&bar_dw[1], ph_dw1); ph_dw1 ^= 1; } else { mbar_wait_backoff(&bar_dw[0], ph_dw0); ph_dw0 ^= 1; }
       tc_fence_after();
       if (warp == NWE) K3X_MARK(jt, 10);
       float gw[CWT];
@@ -1531,89 +1195,6 @@ __global__ void __launch_bounds__(Tc2Cfg<CWT>::NTHR, 1) dec_out_train_tc2_kernel
   if (warp == 0) K3X_MARK(39, 8);
   if (warp == 2 * NWE) tmem_dealloc(tmem, TMEM_COLS);
   trace_mark(TR_K3, 1);
-}
-
-// ---------------------------------------------------------------------------------------------
-// scores kernel (predict): out[b, v] = logit or sigmoid(logit); loops over batch chunks per tile
-// ---------------------------------------------------------------------------------------------
-template <int SPLIT>
-__global__ void __launch_bounds__(NT, 1) dec_out_scores_tc_kernel(const float* __restrict__ h2, int B, int H,
-                                                                  const float* __restrict__ Wd3,
-                                                                  const float* __restrict__ bd3, int Vloc,
-                                                                  int apply_sigmoid, float* __restrict__ out,
-                                                                  int64_t ldo) {
-  constexpr int split = SPLIT;
-  extern __shared__ __align__(1024) unsigned char smem[];
-  __shared__ uint64_t bar_mma;
-  __shared__ uint32_t tmem_base_s;
-  const Geom g = make_geom(H);
-  unsigned char* hb_hi = smem;
-  unsigned char* hb_lo = hb_hi + g.hb_bytes;
-  unsigned char* wb_hi = hb_lo + g.hb_bytes;
-  unsigned char* wb_lo = wb_hi + g.wb_bytes;
-  const bool with_lo = (split == 3);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int q4 = warp & 3, cpart = warp >> 2;
-  const int n_tiles = (Vloc + TN - 1) / TN;
-  const int n_chunks = (B + BM - 1) / BM;
-  if (warp == 0) tmem_alloc(&tmem_base_s, 32);
-  if (tid == 0) {
-    mbar_init(&bar_mma, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = tmem_base_s;
-  const uint32_t lane_addr = tmem + ((uint32_t)(q4 * 32) << 16);
-  uint32_t phase = 0;
-  const uint32_t idesc_g1 = make_idesc(BM, TN, 0, 0);
-  const SmemOp op_hb = make_op(hb_hi, hb_lo, CORE, g.hb_sbo, 2 * CORE);
-  const SmemOp op_wb = make_op(wb_hi, wb_lo, CORE, g.wb_sbo, 2 * CORE);
-  WChunk wc[WCH];
-  make_wchunks(wc, g);
-  // batch chunks are the outer loop of a CTA (blockIdx.y strides over them): the H2' chunk is built once
-  for (int chunk = blockIdx.y; chunk < n_chunks; chunk += gridDim.y) {
-    const int b0 = chunk * BM, nb = min(BM, B - b0);
-    __syncthreads();
-    fill_hb(hb_hi, hb_lo, g, h2, b0, nb, with_lo);
-    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      const int v0 = tile * TN, nv = min(TN, Vloc - v0);
-      float4 wr[WCH];
-      load_w_regs(wr, wc, Wd3, bd3, H, v0, nv);
-      store_w_regs(wr, wc, wb_hi, wb_lo, nullptr, nullptr, with_lo);
-      fence_async_smem();
-      __syncthreads();
-      if (warp == 0) {
-        tc_fence_after();
-        if (elect_one()) {
-          issue_gemm<SPLIT>(tmem, op_hb, op_wb, g.Kp / 8, idesc_g1, 0u);
-          mma_commit(&bar_mma);
-        }
-        __syncwarp();
-      }
-      mbar_wait(&bar_mma, phase);
-      phase ^= 1;
-      tc_fence_after();
-      float z[CW];
-      tmem_ld8(lane_addr + cpart * CW, z);
-      const int brow = q4 * 32 + lane;
-      if (brow < nb) {
-        float* orow = out + (size_t)(b0 + brow) * ldo + v0 + cpart * CW;
-#pragma unroll
-        for (int j = 0; j < CW; ++j) {
-          if (cpart * CW + j < nv) {
-            float s = z[j];
-            if (apply_sigmoid) s = 1.0f / (1.0f + expf(-s));
-            orow[j] = s;
-          }
-        }
-      }
-      tc_fence_before();
-      __syncthreads();
-    }
-  }
-  if (warp == 0) tmem_dealloc(tmem, 32);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1752,7 +1333,7 @@ __global__ void __launch_bounds__(NT, 1) tc_selftest_kernel(int mode_in, const f
     }
     __syncwarp();
   }
-  mbar_wait(&bar_mma, 0);
+  mbar_wait_backoff(&bar_mma, 0);
   tc_fence_after();
   const int ncols = (mode == 2 || mode == 6) ? g.Np : TN;
   const uint32_t tsrc = (mode == 1) ? TM_Z : ((mode == 2 || mode == 6) ? TM_DH : TM_DW);
@@ -1767,267 +1348,7 @@ __global__ void __launch_bounds__(NT, 1) tc_selftest_kernel(int mode_in, const f
   if (warp == 0) tmem_dealloc(tmem, TMEM_COLS);
 }
 
-// ---------------------------------------------------------------------------------------------
-// K5: pipelined scores kernel with a selection epilogue (predict + ranking without the [B,V] round trip).
-//
-// One CTA = one chunk of 128 query rows x a strided subset of 128-item tiles.  The A operand (the H2' chunk, hi and lo
-// parts) lives in TMEM for the whole chunk (ts-form MMAs: lane = query row, column = k): an SS-mode M128 MMA would
-// re-read 4 KB of A from shared memory per instruction, more than the 128 B/cycle shared memory delivers.
-// Warp 16 issues the MMAs (39 x M128.N128.K8 per tile with the 3xTF32 split); warps 0-15 are loaders (W' tile -> tf32
-// hi/lo K-major operand, two 106 KB shared-memory stages) and epilogue (two 128-column TMEM accumulator buffers):
-// while tile i is drained and tile i+2 is staged, the tensor pipe runs tile i+1.  Per stage s one mbarrier pair:
-// ready[s] (one arrival per loader warp: stage filled AND accumulator s drained) and mma[s] (tcgen05.commit: logits
-// of the tile in TMEM, stage s free again).
-// Epilogues: DENSE (scores, optionally sigmoid, to out[b, col]; col = item, or the visit order for the threshold
-// sample) and FILTER (z > tau[b]: append (z, item) to a private sub-list of the row; ~0.07 % of the elements).
-// Replaces the dense lin3 + sigmoid of predict (aae.py:866-868) and the front half of remove_non_missing + argtopk
-// (evaluation.py:183-199, 20-58).
-// ---------------------------------------------------------------------------------------------
-// (Staging the W' tiles with cp.async straight into the hi operand half was measured slower with the 3xTF32 split --
-// 2.59 vs 2.18 ms at V=2M / B=1000: the lo pass then sits between the epilogue and the stage hand-over -- and removed.)
-constexpr int PN = 128;                // items per tile
-constexpr int P_NWE = 16;              // loader / epilogue warps
-constexpr int P_NT = 32 * P_NWE + 32;  // + the MMA warp
-constexpr int P_CW = PN / 4;           // accumulator columns per epilogue thread (4 warps per TMEM lane quarter)
-constexpr int P_WCH = 7;               // 16-byte W' chunks per loader thread (8 rows x <= 28 column groups per warp)
-constexpr uint32_t P_T_AHI = 256, P_T_ALO = 384, P_TMEM_COLS = 512;   // TMEM: accumulators 2 x PN | A hi (Kp <= 128) | A lo
-
-struct SelArgs {
-  const float* h2; int B, H;
-  const float* Wd3; const float* bd3; int Vloc, v_begin;
-  int tile_stride, n_sel;              // tiles visited: j * tile_stride, j < n_sel
-  int filter;                          // 0: dense scores, 1: threshold filter
-  float* out; long long ldo; int out_by_visit, apply_sigmoid;
-  // filter: row b owns gridDim.x * 4 private sub-lists (one per CTA column x and 32-column part of the tile) of cap_sub
-  // slots; sub-list counters live in registers (one writer each: no atomics, deterministic order) and are stored to
-  // cnt[b * nsub + sub] at the end of the chunk (a count above cap_sub = overflow)
-  const float* tau; int tau_stride; int32_t* cnt; float* cand_val; int32_t* cand_idx; int cap_sub;
-};
-
-// Loader mapping (16 warps, 128 rows x Kp/4 <= 28 column groups of 16 bytes): warp w owns the 8 rows 8w .. 8w+7 and
-// all column groups; lane & 7 = row inside the group, column groups (lane >> 3) + 4 j.  One warp-wide load touches
-// 8 rows x 64 contiguous bytes (8-16 cache lines) instead of 32 rows x 16 bytes (32 lines): with a row-per-lane
-// mapping the kernel was bound by the L1TEX tag stage (ncu: l1tex throughput 85 %, 31 sectors per request).  A
-// quarter warp writes 8 consecutive rows of one column group = one 128-byte core matrix: conflict-free.
-// All per-thread offsets are tile-invariant and computed once (goff: float offset inside the tile's rows, -1 = bias
-// column, -2 = unused; soff: byte offset inside a stage half).
-struct PChunks {
-  int goff[P_WCH];
-  uint32_t soff[P_WCH];
-};
-__device__ __forceinline__ void p_load_w(float4* wr, const PChunks& pc, const float* __restrict__ wtile,
-                                         const float* __restrict__ btile, bool rv) {
-#pragma unroll
-  for (int j = 0; j < P_WCH; ++j) {
-    float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (rv) {
-      if (pc.goff[j] >= 0) x = __ldg(reinterpret_cast<const float4*>(wtile + pc.goff[j]));
-      else if (pc.goff[j] == -1) x.x = __ldg(btile);
-    }
-    wr[j] = x;
-  }
-}
-__device__ __forceinline__ void p_store_w(const float4* wr, const PChunks& pc, unsigned char* hi, unsigned char* lo,
-                                          bool with_lo) {
-#pragma unroll
-  for (int j = 0; j < P_WCH; ++j) {
-    if (pc.goff[j] == -2) continue;
-    const float4 x = wr[j];
-    const float4 h = make_float4(tf32_hi(x.x), tf32_hi(x.y), tf32_hi(x.z), tf32_hi(x.w));
-    *reinterpret_cast<float4*>(hi + pc.soff[j]) = h;
-    if (with_lo) *reinterpret_cast<float4*>(lo + pc.soff[j]) = make_float4(x.x - h.x, x.y - h.y, x.z - h.z, x.w - h.w);
-  }
-}
-
-template <int SPLIT>
-__global__ void __launch_bounds__(P_NT, 1) dec_out_select_kernel(SelArgs a) {
-  extern __shared__ __align__(1024) unsigned char smem[];
-  __shared__ uint64_t bar_mma[2], bar_ready[2];
-  __shared__ uint32_t tmem_base_s;
-  constexpr bool with_lo = (SPLIT == 3);
-  const Geom g = make_geom(a.H);
-  const uint32_t wb_bytes = (PN / 8) * g.wb_sbo;
-  unsigned char* wst = smem;                       // stage s: hi at wst + 2*s*wb_bytes, lo right after
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int ncg = g.Kp / 4;
-  const int n_chunks = (a.B + BM - 1) / BM;
-  const int n_my = ((int)blockIdx.x < a.n_sel) ? (a.n_sel - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
-  for (uint32_t q = tid; q < 4u * wb_bytes / 16u; q += P_NT) reinterpret_cast<float4*>(wst)[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (warp == P_NWE) tmem_alloc(&tmem_base_s, P_TMEM_COLS);
-  if (tid == 0) {
-    mbar_init(&bar_mma[0], 1);
-    mbar_init(&bar_mma[1], 1);
-    mbar_init(&bar_ready[0], P_NWE);
-    mbar_init(&bar_ready[1], P_NWE);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = tmem_base_s;
-  const uint32_t idesc = make_idesc(BM, PN, 0, 0);
-  uint32_t ph0 = 0, ph1 = 0;                       // parity of the barrier this role waits on, per stage
-  for (int chunk = blockIdx.y; chunk < n_chunks; chunk += gridDim.y) {
-    const int b0 = chunk * BM, nb = min(BM, a.B - b0);
-    __syncthreads();                               // the previous chunk is drained: the A operand may be rebuilt
-    if (warp < P_NWE) {
-      // H2' chunk -> TMEM (A operand of every MMA of this chunk: lane = query row, column = k; hi and lo parts).
-      // A from TMEM instead of shared memory: an SS-mode M128 x K8 tf32 MMA reads 4 KB of A per slot on top of B,
-      // more than the 128 B/cycle the shared memory delivers -- with A in shared memory the kernel was feed-bound.
-      const int q4 = warp & 3, cpart = warp >> 2;
-      const uint32_t lane_addr = tmem + ((uint32_t)(q4 * 32) << 16);
-      const int brow = q4 * 32 + lane;
-      for (int c = cpart; c < g.Kp / 8; c += 4) {
-        float hi[8], lo[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int kk = c * 8 + j;
-          float x = 0.f;
-          if (brow < nb) x = (kk < a.H) ? __ldg(a.h2 + (size_t)(b0 + brow) * a.H + kk) : (kk == a.H ? 1.0f : 0.f);
-          hi[j] = tf32_hi(x);
-          lo[j] = x - hi[j];
-        }
-        tmem_st8(lane_addr + P_T_AHI + c * 8, hi);
-        if (with_lo) tmem_st8(lane_addr + P_T_ALO + c * 8, lo);
-      }
-      tmem_st_wait();
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    if (warp == P_NWE) {
-      // ================= MMA issuer =================
-      const SmemOp op_w0 = make_op(wst, wst + wb_bytes, CORE, g.wb_sbo, 2 * CORE);
-      const SmemOp op_w1 = make_op(wst + 2 * wb_bytes, wst + 3 * wb_bytes, CORE, g.wb_sbo, 2 * CORE);
-      for (int it = 0; it < n_my; ++it) {
-        const int s = it & 1;
-        mbar_wait(&bar_ready[s], s ? ph1 : ph0);
-        if (s) ph1 ^= 1; else ph0 ^= 1;
-        tc_fence_after();
-        if (elect_one()) {
-          issue_gemm_ts<SPLIT>(tmem + (uint32_t)(s * PN), tmem + P_T_AHI, tmem + P_T_ALO, s ? op_w1 : op_w0, g.Kp / 8,
-                               idesc, 0u);
-          mma_commit(&bar_mma[s]);
-        }
-        __syncwarp();
-      }
-    } else {
-      // ================= loaders + epilogue =================
-      const int q4 = warp & 3, cpart = warp >> 2;
-      const uint32_t lane_addr = tmem + ((uint32_t)(q4 * 32) << 16);
-      const int brow = q4 * 32 + lane;
-      const bool rowv = brow < nb;
-      float tau = __int_as_float(0x7f800000);
-      if (a.filter && rowv) tau = a.tau[(size_t)(b0 + brow) * a.tau_stride];
-      const int nsub = (int)gridDim.x * 4, sub = (int)blockIdx.x * 4 + cpart;
-      const size_t sub_base = ((size_t)(b0 + brow) * nsub + sub) * (size_t)a.cap_sub;
-      int my_cnt = 0;
-      // loader role of this thread
-      const int lrow = warp * 8 + (lane & 7);
-      PChunks pc;
-#pragma unroll
-      for (int j = 0; j < P_WCH; ++j) {
-        const int cg = (lane >> 3) + 4 * j, c = cg * 4;
-        pc.goff[j] = (cg < ncg) ? ((c + 3 < a.H) ? lrow * a.H + c : (c == a.H ? -1 : -3)) : -2;
-        pc.soff[j] = (uint32_t)(lrow >> 3) * g.wb_sbo + (uint32_t)cg * CORE + (uint32_t)(lrow & 7) * 16u;
-      }
-      const int tile_step = (int)gridDim.x * a.tile_stride * PN;           // items between two tiles of this CTA
-      const int v_first = (int)blockIdx.x * a.tile_stride * PN;
-      auto load_tile = [&](float4* wr, int v0) {
-        p_load_w(wr, pc, a.Wd3 + (size_t)v0 * a.H, a.bd3 + v0 + lrow, v0 + lrow < a.Vloc);
-      };
-      float4 wr[P_WCH];
-      for (int p = 0; p < 2 && p < n_my; ++p) {
-        load_tile(wr, v_first + p * tile_step);
-        p_store_w(wr, pc, wst + 2 * p * wb_bytes, wst + (2 * p + 1) * wb_bytes, with_lo);
-        fence_async_smem();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&bar_ready[p]);
-      }
-      if (n_my > 2) load_tile(wr, v_first + 2 * tile_step);
-      for (int i = 0; i < n_my; ++i) {
-        const int s = i & 1;
-        const int v0 = v_first + i * tile_step;
-        mbar_wait(&bar_mma[s], s ? ph1 : ph0);       // logits of tile i in TMEM buffer s, stage s free again
-        if (s) ph1 ^= 1; else ph0 ^= 1;
-        tc_fence_after();
-        uint32_t zr[P_CW];
-        TmemIO<16>::ld_issue(lane_addr + (uint32_t)(s * PN + cpart * P_CW), zr);
-        TmemIO<16>::ld_issue(lane_addr + (uint32_t)(s * PN + cpart * P_CW + 16), zr + 16);
-        TmemIO<16>::ld_wait(zr);
-        TmemIO<16>::ld_wait(zr + 16);
-        tc_fence_before();
-        if (i + 2 < n_my) {
-          p_store_w(wr, pc, wst + 2 * s * wb_bytes, wst + (2 * s + 1) * wb_bytes, with_lo);
-          fence_async_smem();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bar_ready[s]);
-          if (i + 3 < n_my) load_tile(wr, v0 + 3 * tile_step);
-        }
-        // ---- epilogue of tile i
-        const int c0 = cpart * P_CW;
-        const int vm = a.Vloc - v0 - c0;                         // valid columns among this thread's 32
-        if (a.filter) {
-          float zmax = __uint_as_float(zr[0]);
-#pragma unroll
-          for (int j = 1; j < P_CW; ++j) zmax = fmaxf(zmax, __uint_as_float(zr[j]));
-          if (zmax > tau) {
-#pragma unroll
-            for (int j = 0; j < P_CW; ++j) {
-              const float z = __uint_as_float(zr[j]);
-              if (z > tau && j < vm) {
-                if (my_cnt < a.cap_sub) {
-                  a.cand_val[sub_base + my_cnt] = z;
-                  a.cand_idx[sub_base + my_cnt] = a.v_begin + v0 + c0 + j;
-                }
-                ++my_cnt;
-              }
-            }
-          }
-        } else if (rowv) {
-          const int colbase = a.out_by_visit ? ((int)blockIdx.x + i * (int)gridDim.x) * PN : v0;
-          float* orow = a.out + (size_t)(b0 + brow) * a.ldo + colbase + c0;
-          if (vm >= P_CW && ((reinterpret_cast<uintptr_t>(orow) & 15) == 0)) {
-#pragma unroll
-            for (int j = 0; j < P_CW; j += 4) {
-              float4 o;
-              o.x = __uint_as_float(zr[j]); o.y = __uint_as_float(zr[j + 1]);
-              o.z = __uint_as_float(zr[j + 2]); o.w = __uint_as_float(zr[j + 3]);
-              if (a.apply_sigmoid) {
-                o.x = 1.0f / (1.0f + expf(-o.x)); o.y = 1.0f / (1.0f + expf(-o.y));
-                o.z = 1.0f / (1.0f + expf(-o.z)); o.w = 1.0f / (1.0f + expf(-o.w));
-              }
-              __stcs(reinterpret_cast<float4*>(orow + j), o);
-            }
-          } else {
-#pragma unroll
-            for (int j = 0; j < P_CW; ++j) {
-              if (j < vm) {
-                float sc = __uint_as_float(zr[j]);
-                if (a.apply_sigmoid) sc = 1.0f / (1.0f + expf(-sc));
-                orow[j] = sc;
-              }
-            }
-          }
-        }
-      }
-      if (a.filter && rowv) a.cnt[(size_t)(b0 + brow) * nsub + sub] = my_cnt;
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == P_NWE) tmem_dealloc(tmem, P_TMEM_COLS);
-}
-
 }  // namespace tc
-
-static bool tc_supported(int B, int H, const char* what) {
-  if ((H & 3) != 0 || H + 1 > 128) {
-    set_error("%s: tensor-core kernel needs n_hidden %% 4 == 0 and n_hidden <= 124 (got %d); use impl=simt", what, H);
-    return false;
-  }
-  return true;
-}
 
 // smem of the pipelined kernel: Hb hi/lo (round8(B) rows) + Wb hi/lo + Wtb hi/lo + Dtb hi/lo + E2 stage
 static size_t tc2_smem_bytes(const tc::Geom& g, int B) {
@@ -2136,62 +1457,6 @@ int dec_out_train_tc(const float* h2, int B, int H, float* Wd3, float* bd3, floa
                                   (float)(1.0 / n_total), st, dh2, loss_sum);
   return check_launch("dec_out_train(tc)");
 }
-
-// grid of the K5 kernel for B query rows and n_sel tiles: y = chunks of 128 rows, x = CTAs sharing a chunk
-void dec_out_select_grid(int B, int n_sel, int* gx, int* gy) {
-  const int n_chunks = (B + tc::BM - 1) / tc::BM;
-  *gy = std::min(n_chunks, sm_count());
-  *gx = std::max(1, std::min(n_sel, sm_count() / *gy));
-}
-
-// K5 launcher: dense scores (filter == 0) or threshold filter (filter == 1) over the tiles j * tile_stride, j < n_sel.
-int dec_out_select_tc(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int v_begin,
-                      int tile_stride, int n_sel, int filter, float* out, int64_t ldo, int out_by_visit,
-                      int apply_sigmoid, const float* tau, int tau_stride, int32_t* cnt, float* cand_val,
-                      int32_t* cand_idx, int cap, int split, cudaStream_t s) {
-  if (!tc_supported(B, H, "dec_out_select")) return AAE_E_UNSUPPORTED;
-  tc::Geom g = tc::make_geom(H);
-  const size_t smem = 4 * (size_t)(tc::PN / 8) * g.wb_sbo + 256;
-  auto kern = (split == 3) ? tc::dec_out_select_kernel<3> : tc::dec_out_select_kernel<1>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) {
-    set_error("dec_out_select: smem %zu: %s", smem, cudaGetErrorString(e));
-    return AAE_E_CUDA;
-  }
-  tc::SelArgs a;
-  a.h2 = h2; a.B = B; a.H = H; a.Wd3 = Wd3; a.bd3 = bd3; a.Vloc = Vloc; a.v_begin = v_begin;
-  a.tile_stride = tile_stride; a.n_sel = n_sel; a.filter = filter;
-  a.out = out; a.ldo = ldo; a.out_by_visit = out_by_visit; a.apply_sigmoid = apply_sigmoid;
-  a.tau = tau; a.tau_stride = tau_stride; a.cnt = cnt; a.cand_val = cand_val; a.cand_idx = cand_idx; a.cap_sub = cap;
-  int gx, gy;
-  dec_out_select_grid(B, n_sel, &gx, &gy);
-  kern<<<dim3(gx, gy), tc::P_NT, smem, s>>>(a);
-  return check_launch("dec_out_select");
-}
-
-int dec_out_scores_tc(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int apply_sigmoid,
-                      float* out, int64_t ldo, int split, cudaStream_t s) {
-  if (!tc_supported(B, H, "dec_out_scores")) return AAE_E_UNSUPPORTED;
-  if (split < 10)
-    return dec_out_select_tc(h2, B, H, Wd3, bd3, Vloc, 0, 1, (Vloc + tc::PN - 1) / tc::PN, 0, out, ldo, 0, apply_sigmoid,
-                             nullptr, 0, nullptr, nullptr, nullptr, 0, split, s);
-  split -= 10;
-  tc::Geom g = tc::make_geom(H);
-  size_t smem = 2 * ((size_t)g.hb_bytes + g.wb_bytes) + 256;
-  auto kern = (split == 3) ? tc::dec_out_scores_tc_kernel<3> : tc::dec_out_scores_tc_kernel<1>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) {
-    set_error("dec_out_scores(tc): smem %zu: %s", smem, cudaGetErrorString(e));
-    return AAE_E_CUDA;
-  }
-  int n_tiles = (Vloc + tc::TN - 1) / tc::TN;
-  int n_chunks = (B + tc::BM - 1) / tc::BM;
-  int gy = std::min(n_chunks, sm_count());
-  int gx = std::max(1, std::min(n_tiles, sm_count() / gy));
-  kern<<<dim3(gx, gy), tc::NT, smem, s>>>(h2, B, H, Wd3, bd3, Vloc, apply_sigmoid, out, ldo);
-  return check_launch("dec_out_scores(tc)");
-}
-
 }  // namespace aae
 
 extern "C" int aae_tc_selftest(int mode, const float* A, const float* Bm, float* D, int split, void* stream) {

@@ -14,7 +14,7 @@
 #include <float.h>
 #include <math.h>
 #include <algorithm>
-#include "common.cuh"
+#include "dec_out.cuh"
 
 namespace aae {
 
@@ -461,24 +461,12 @@ __global__ void __launch_bounds__(KTH_THREADS) row_kth_approx_kernel(const float
   if (threadIdx.x == 0) tau[blockIdx.x] = key2f((uint32_t)(buf[min(J, KTH_THREADS * KTH_KEEP) - 1] >> 32));
 }
 
-int dec_out_select_tc(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int v_begin,
-                      int tile_stride, int n_sel, int filter, float* out, int64_t ldo, int out_by_visit,
-                      int apply_sigmoid, const float* tau, int tau_stride, int32_t* cnt, float* cand_val,
-                      int32_t* cand_idx, int cap, int split, cudaStream_t s);
-
 // Plan of the fused predict + top-k path for one (Vloc, k): sample tiles, threshold rank, candidate capacity.
-void dec_out_select_grid(int B, int n_sel, int* gx, int* gy);
-
 struct TopkPlan {
   int n_tiles, n_samp, stride, S, T, J, cap;
   int nsub, cap_sub;       // private candidate sub-lists per row (one per CTA column and 16-column tile part)
   bool ok;
 };
-void dec_out_select2_grid(int B, int n_sel, int* gx, int* gy);
-int dec_out_select2(const float* h2, int B, int H, const float* Wp, int Vloc, int v_begin, int tile_stride, int n_sel,
-                    int filter, float* out, int64_t ldo, int out_by_visit, const float* tau, int32_t* cnt,
-                    int32_t* cand_idx, int cap_sub, cudaStream_t s);
-bool select2_supported(int H);
 
 static TopkPlan make_plan(int B, int Vloc, int k, bool v2 = false) {
   TopkPlan p;

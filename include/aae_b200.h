@@ -225,7 +225,9 @@ int aae_dec_out_train_ws(const float* h2, int B, int H, float* Wd3, float* bd3, 
                          int64_t work_floats, void* stream);
 
 /* ---- predict (aae.py:840-870) --------------------------------------------------------------- */
-/* out[b, v] = logit or sigmoid(logit) for local items; ldo = row pitch of out in floats. */
+/* out[b, v] = logit or sigmoid(logit) for local items; ldo = row pitch of out in floats.
+ * impl: 0 = fp32 CUDA-core kernel, 1 = tcgen05 3xTF32 (fp32-accurate), 2 = tcgen05 single-pass TF32; 3 and 4 score as
+ * 1 and 2 (the choice of kernel they make in aae_dec_out_train exists only for training); any other value: AAE_E_ARG. */
 int aae_dec_out_scores(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc,
                        int apply_sigmoid, float* out, int64_t ldo, int impl, void* stream);
 /* Ranking tail = remove_non_missing + argtopk (evaluation.py:183-199, 20-58) without the dense

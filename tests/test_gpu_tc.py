@@ -124,7 +124,7 @@ def test_tc_scores_match_fp32_kernel(B, V):
     b = (torch.rand(V, generator=g) - 0.5).cuda()
     h2 = torch.relu(torch.randn(B, H, generator=g)).cuda()
     outs = []
-    for impl in (0, 1):
+    for impl in (0, 1, 3):
         o = torch.zeros(B, V, device="cuda")
         N.call("aae_dec_out_scores", N.ptr(h2), B, H, N.ptr(W), N.ptr(b), V, 0, N.ptr(o), V, impl, None)
         torch.cuda.synchronize()
@@ -132,3 +132,4 @@ def test_tc_scores_match_fp32_kernel(B, V):
     want = h2.cpu().double() @ W.cpu().double().t() + b.cpu().double()
     assert (outs[0] - want).abs().max() < 2e-5
     assert (outs[1] - want).abs().max() < 2e-5
+    assert torch.equal(outs[2], outs[1])   # impl 3 scores as impl 1
