@@ -40,6 +40,11 @@ class AaePeers(C.Structure):
     _fields_ = [("base", P * 8), ("rank", I), ("world", I)]
 
 
+class AaeRankFilter(C.Structure):
+    """Mirror of ``aae_rank_filter``: column -> global id table and per-row exclusion CSR of a filtered ranking."""
+    _fields_ = [("item_ids", P), ("excl_indptr", P), ("excl_indices", P)]
+
+
 class StepState(C.Structure):
     """Mirror of ``aae_step_state`` (device resident; used for size and for debugging reads)."""
     _fields_ = [("t", C.c_int32), ("rng_step", C.c_uint32), ("step_size_gen", F), ("step_size_reg", F),
@@ -83,6 +88,12 @@ _SIGS = {
     "aae_pad_weights": (I, [P, P, I, I, P, P, P]),
     "aae_predict_topk2_work_bytes": (I64, [I, I, I, I]),
     "aae_predict_topk2": (I, [P, I, I, P, P, P, P, I, I, P, P, I, P, I64, P, P, P, P]),
+    "aae_gather_item_rows": (I, [P, P, I, I, I, P, I, P, P, P, P]),
+    "aae_masked_topk_filtered": (I, [P, I64, I, I, I, P, P, I, P, P, P, P, C.POINTER(AaeRankFilter)]),
+    "aae_predict_topk_filtered": (I, [P, I, I, P, P, I, I, P, P, I, I, P, I64, P, P, P, P,
+                                      C.POINTER(AaeRankFilter)]),
+    "aae_predict_topk2_filtered": (I, [P, I, I, P, P, P, P, I, I, P, P, I, P, I64, P, P, P, P,
+                                       C.POINTER(AaeRankFilter)]),
     "aae_tc_selftest": (I, [I, P, P, P, I, P]),
     "aae_upload_batch": (I, [P, P, I, I, P, P, P]),
     "aae_batch_gather": (I, [P, P, P, I64, I, P, P, P, I, P, P]),
@@ -138,7 +149,8 @@ def last_error():
 
 
 # kernels launched per entry point (for the bench's gpu_launches claim); memcpy-only calls count 0
-KERNELS = {"aae_upload_batch": 0, "aae_w1_sweep_blocked": 2, "aae_batch_gather": 2, "aae_batch_corrupt": 2, "aae_rank_counts": 3, "aae_masked_topk": 2, "aae_predict_topk": 6, "aae_predict_topk2": 8, "aae_trace_set": 0, "aae_trace_slots": 0,
+KERNELS = {"aae_upload_batch": 0, "aae_w1_sweep_blocked": 2, "aae_batch_gather": 2, "aae_batch_corrupt": 2, "aae_rank_counts": 3, "aae_masked_topk": 2, "aae_predict_topk": 6, "aae_predict_topk2": 8, "aae_masked_topk_filtered": 3, "aae_predict_topk_filtered": 6,
+           "aae_predict_topk2_filtered": 8, "aae_trace_set": 0, "aae_trace_slots": 0,
            "aae_peer_alloc": 0, "aae_peer_open": 0, "aae_peer_close": 0, "aae_peer_free": 0, "aae_peer_error": 0}
 TRACE_NAMES = ("batch_prepare", "w1_sweep_untouched", "ae_fwd", "dec_out_train", "ae_bwd", "ae_wgrad", "w1_rows_update_1",
                "disc_phase", "disc_wgrad", "gen_phase", "gen_wgrad", "w1_rows_update_2", "step_finish", "bag_fwd", "w1_catchup")

@@ -22,6 +22,7 @@ import torch
 from .base import Recommender
 from .condition import _check_conditions, CondAdapter
 from .engine import AAEEngine
+from .filters import RankFilter
 
 torch.manual_seed(42)   # aae.py:27 -- the reference seeds the CPU generator at import
 TINY = 1e-12
@@ -493,19 +494,34 @@ class AdversarialAutoEncoder(object):
         eng.check_exchange()
         return out
 
-    def predict_topk(self, X, k, condition_data=None, mask_known=True, return_scores=False, shard="items"):
+    def predict_topk(self, X, k, condition_data=None, mask_known=True, return_scores=False, shard="items",
+                     items=None, exclude=None):
         """Top-k unknown items per row = argtopk(remove_non_missing(predict(X), X), k)[1]
         (evaluation.py:183-199, 20-58) without materialising [n, n_items] on the host.
 
         Multi-GPU: ``shard='items'`` ranks every query against the local item shard and merges the per-shard lists
         (one all-gather per batch); ``shard='sets'`` gives every rank a full-weight replica (built once) and its own
-        slice of the query rows -- no communication in the query loop; the slices are exchanged at the end."""
+        slice of the query rows -- no communication in the query loop; the slices are exchanged at the end.
+
+        Candidate restriction (both absent: the unrestricted ranking above):
+          ``items``   eligible items: 1-D array of item ids in [0, n_items) (duplicates allowed) or a boolean mask of
+                      length n_items (a block list is ``items=~blocked``); only these are ranked.
+          ``exclude`` scipy sparse [n, n_items]: the nonzero entries of row i are never returned for row i.
+        Semantics: ineligible items and excluded (row, item) pairs are never returned.  With ``mask_known`` a known
+        item that is eligible and not excluded ranks below every unknown one (score -FLT_MAX, as without a filter); a
+        known item that is ineligible or excluded is not returned.  Ties go to the lower item id.  A row with fewer
+        than k returnable items is padded at the end with item id -1 and score -inf.  ``k=None`` (or k > MAX_TOPK)
+        gives the full ranking of the eligible items: A columns for k=None (A = number of eligible items), min(k, A)
+        otherwise, padded the same way; item-sharded full rankings raise as without a filter.  Ids out of range, a mask of the wrong length or an ``exclude`` of the wrong
+        shape raise ValueError.  The eligible rows of the output layer are ranked as a compact copy cached on the
+        engine (rebuilt when the eligible set or the weights change)."""
+        filt = RankFilter.build(self.engine.V, X.shape[0], items, exclude)
         if k is None or k > self.MAX_TOPK:
             # argtopk's k=None / k >= size branch (evaluation.py:48-52): the full ranking of every row
             return self._full_ranking(X, eng_k=k, condition_data=condition_data, mask_known=mask_known,
-                                      return_scores=return_scores)
+                                      return_scores=return_scores, filt=filt)
         if shard == "sets" and self.engine.world > 1:
-            return self._predict_topk_set_sharded(X, k, condition_data, mask_known, return_scores)
+            return self._predict_topk_set_sharded(X, k, condition_data, mask_known, return_scores, filt)
         eng = self.engine
         n = X.shape[0]
         kk = min(k, eng.V)
@@ -515,7 +531,7 @@ class AdversarialAutoEncoder(object):
         # (the fused path keeps no [B,V] matrix, so the batch only sizes the candidate lists)
         pb = max(self.batch_size, self.predict_batch_size)
         for start, end, B in self._iter_batches(X, condition_data, batch_size=pb):
-            i, v = eng.topk(B, kk, mask_known=mask_known)
+            i, v = eng.topk(B, kk, mask_known=mask_known, filt=None if filt is None else filt.rows(start, end))
             idx[start:end] = i.cpu().numpy()
             if return_scores:
                 val[start:end] = v.cpu().numpy()
@@ -526,7 +542,7 @@ class AdversarialAutoEncoder(object):
 
     MAX_TOPK = 4096       # envelope of the selection kernels (aae_masked_topk / aae_predict_topk2)
 
-    def _full_ranking(self, X, eng_k, condition_data, mask_known, return_scores):
+    def _full_ranking(self, X, eng_k, condition_data, mask_known, return_scores, filt=None):
         """All items of every row in descending order of remove_non_missing(predict(X), X) -- ``argtopk(.., k=None)``
         (evaluation.py:48-52), or its first ``k`` columns for a k beyond the selection kernels' envelope.  The [B, V]
         logit matrix is built by the decoder kernel and sorted on the device (known items last, ties by lower item id);
@@ -536,6 +552,8 @@ class AdversarialAutoEncoder(object):
         if eng.world > 1:
             raise NotImplementedError("full rankings (k=None or k > %d) on item shards: use evaluate_topk for unbounded "
                                       "metrics, or a single-GPU / set-sharded replica" % self.MAX_TOPK)
+        if filt is not None:
+            return self._full_ranking_filtered(X, eng_k, condition_data, mask_known, return_scores, filt)
         n, V = X.shape[0], eng.V
         kk = V if eng_k is None else min(eng_k, V)
         idx = np.empty((n, kk), dtype=np.int64)
@@ -555,7 +573,46 @@ class AdversarialAutoEncoder(object):
                 val[start:end] = v[:, :kk].cpu().numpy()
         return (idx, val) if return_scores else idx
 
-    def _predict_topk_set_sharded(self, X, k, condition_data, mask_known, return_scores):
+    def _full_ranking_filtered(self, X, eng_k, condition_data, mask_known, return_scores, filt):
+        """``_full_ranking`` under a candidate filter: the [B, A] logits of the eligible items only (compact copy of
+        the output layer) are sorted on the device and mapped back to item ids; known items score -FLT_MAX (below
+        every unknown one), excluded ones -inf, which come out as the (-1, -inf) padding at the end of the row."""
+        eng = self.engine
+        n, V = X.shape[0], eng.V
+        A = filt.n_eligible(V)
+        kk = A if eng_k is None else min(eng_k, A)
+        idx = np.empty((n, kk), dtype=np.int64)
+        val = np.empty((n, kk), dtype=np.float32) if return_scores else None
+        for start, end, B in self._iter_batches(X, condition_data):
+            if filt.items is None:
+                sc = eng.scores(B, torch.empty(B, V, dtype=torch.float32, device=eng.dev), apply_sigmoid=False)
+                ids = torch.arange(V, dtype=torch.int32, device=eng.dev)
+            else:
+                sc, ids = eng.compact_scores(B, filt.items)
+            ids = ids.long()
+
+            def fill(indptr, indices, value):
+                ip = torch.as_tensor(np.asarray(indptr, dtype=np.int64), device=eng.dev)
+                g = torch.as_tensor(np.asarray(indices, dtype=np.int64), device=eng.dev)[: int(ip[-1])]
+                rows = torch.repeat_interleave(torch.arange(B, device=eng.dev), ip[1:] - ip[:-1])
+                col = torch.searchsorted(ids, g).clamp_(max=max(A - 1, 0))
+                hit = ids[col] == g if A else torch.zeros_like(g, dtype=torch.bool)
+                sc[rows[hit], col[hit]] = value
+            if mask_known:
+                fill(eng.indptr[:B + 1].cpu().numpy(), eng.indices[:int(eng.indptr[B])].cpu().numpy(),
+                     -float(np.finfo(np.float32).max))
+            if filt.exclude is not None:
+                ex = filt.exclude[start:end]
+                fill(ex.indptr, ex.indices, -float("inf"))
+            v, i = torch.sort(sc, dim=1, descending=True, stable=True)
+            v, i = v[:, :kk], ids[i[:, :kk]]
+            i.masked_fill_(v == -float("inf"), -1)
+            idx[start:end] = i.cpu().numpy()
+            if return_scores:
+                val[start:end] = v.cpu().numpy()
+        return (idx, val) if return_scores else idx
+
+    def _predict_topk_set_sharded(self, X, k, condition_data, mask_known, return_scores, filt=None):
         import torch.distributed as dist
         eng = self.engine
         if getattr(self, "_replica", None) is None or self._replica_step != eng.steps_done:
@@ -570,8 +627,11 @@ class AdversarialAutoEncoder(object):
             ad = self._cond_adapter()
             cl = [ad.take(c, np.arange(lo, hi)) for c in condition_data]
         main, self.engine = self.engine, self._replica
+        fkw = {} if filt is None else dict(items=filt.items,
+                                           exclude=None if filt.exclude is None else filt.exclude[lo:hi])
         try:
-            out = self.predict_topk(Xl, k, condition_data=cl, mask_known=mask_known, return_scores=return_scores) \
+            out = self.predict_topk(Xl, k, condition_data=cl, mask_known=mask_known, return_scores=return_scores,
+                                    **fkw) \
                 if hi > lo else ((np.zeros((0, min(k, eng.V)), np.int64), np.zeros((0, min(k, eng.V)), np.float32))
                                  if return_scores else np.zeros((0, min(k, eng.V)), np.int64))
         finally:
@@ -684,10 +744,11 @@ class AAERecommender(Recommender):
         condition_data = self._condition_data(test_set, fit=False)
         return self.model.predict(X, condition_data=condition_data)
 
-    def predict_topk(self, test_set, k, mask_known=True):
+    def predict_topk(self, test_set, k, mask_known=True, items=None, exclude=None):
         X = test_set.tocsr()
         condition_data = self._condition_data(test_set, fit=False)
-        return self.model.predict_topk(X, k, condition_data=condition_data, mask_known=mask_known)
+        return self.model.predict_topk(X, k, condition_data=condition_data, mask_known=mask_known, items=items,
+                                       exclude=exclude)
 
     def evaluate_topk(self, test_set, gold, metrics):
         """Ranking metrics of the harness (evaluation.py:70-164, 202-240) on the device: ``gold`` is the sparse

@@ -27,8 +27,9 @@ class Recommender(abc.ABC):
     def predict(self, test_set):
         """Scores [n, n_items] for the item sets of ``test_set`` (float32; higher = more likely missing)."""
 
-    def predict_topk(self, test_set, k, mask_known=True):
-        """Top-k unknown items per set = argtopk(remove_non_missing(predict(test_set), X), k) without the dense matrix."""
+    def predict_topk(self, test_set, k, mask_known=True, items=None, exclude=None):
+        """Top-k unknown items per set = argtopk(remove_non_missing(predict(test_set), X), k) without the dense matrix;
+        ``items`` / ``exclude`` restrict the candidates (``AdversarialAutoEncoder.predict_topk``)."""
         raise NotImplementedError("%s ranks through predict() only" % type(self).__name__)
 
     def evaluate_topk(self, test_set, gold, metrics):

@@ -125,7 +125,7 @@ class DAERecommender(Recommender):
         X = test_set.tocsr()
         return self.dae.predict(X, condition_data=self._condition_data(test_set, fit=False))
 
-    def predict_topk(self, test_set, k, mask_known=True):
+    def predict_topk(self, test_set, k, mask_known=True, items=None, exclude=None):
         X = test_set.tocsr()
         return self.dae.predict_topk(X, k, condition_data=self._condition_data(test_set, fit=False),
-                                     mask_known=mask_known)
+                                     mask_known=mask_known, items=items, exclude=exclude)

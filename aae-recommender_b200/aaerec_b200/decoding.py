@@ -147,6 +147,7 @@ class DecodingRecommender(Recommender):
         X, condition_data = self._query(test_set)
         return self.model.predict(X, condition_data=condition_data)
 
-    def predict_topk(self, test_set, k, mask_known=True):
+    def predict_topk(self, test_set, k, mask_known=True, items=None, exclude=None):
         X, condition_data = self._query(test_set)
-        return self.model.predict_topk(X, k, condition_data=condition_data, mask_known=mask_known)
+        return self.model.predict_topk(X, k, condition_data=condition_data, mask_known=mask_known, items=items,
+                                       exclude=exclude)

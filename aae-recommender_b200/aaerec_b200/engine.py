@@ -99,6 +99,18 @@ class AAEEngine(object):
     def disc_sizes(self):
         return disc_block_sizes(self.H, self.C)
 
+    # Every change of the output layer sets _wp_dirty; it also bumps the weight version that the compact candidate copy
+    # (``_compact``) is checked against.
+    @property
+    def _wp_dirty(self):
+        return self._wp_stale
+
+    @_wp_dirty.setter
+    def _wp_dirty(self, v):
+        self._wp_stale = bool(v)
+        if v:
+            self._wver = getattr(self, "_wver", 0) + 1
+
     def __init__(self, n_items, n_hidden=100, n_code=50, cond_dim=0, gen_lr=1e-3, reg_lr=1e-3,
                  dropout=(.2, .2), prior_scale=None, normalize_inputs=True, device=None,
                  rank=0, world=1, group=None, impl="auto", seed=0, max_batch=128, max_nnz=None,
@@ -148,6 +160,8 @@ class AAEEngine(object):
         self._gwork = None
         self._wp = None             # padded [Vloc,104] copy of the output layer for the TMA-fed predict filter
         self._wp_dirty = True
+        self._cmp = None            # compact [A,H] copy of the shard's eligible rows of the output layer (``_compact``)
+        self._xstage = None         # pinned + device staging of the batch's exclusion CSR (``_upload_exclusions``)
         self._topk_out = None
         f32 = dict(dtype=torch.float32, device=self.dev)
         H, Cc, Cp, Vl = self.H, self.C, self.Cp, max(self.Vloc, 1)
@@ -1077,7 +1091,7 @@ class AAEEngine(object):
         return self._wp, wmax
 
     @_on_device
-    def topk(self, B, k, scratch=None, mask_known=True, fused=None, check=True):
+    def topk(self, B, k, scratch=None, mask_known=True, fused=None, check=True, filt=None, _out=None):
         """Masked top-k of the batch in the device buffers: returns (idx int32 [B,k] global item ids,
         val float32 [B,k] logits), descending.  Item-sharded: local top-k + all-gather + merge.
 
@@ -1086,16 +1100,37 @@ class AAEEngine(object):
         the shape is inside its envelope, else ``aae_predict_topk`` (3xTF32 throughout).  The per-batch status word is
         read back (one 4-byte synchronising copy) and a batch the fused path could not rank exactly is redone through
         the dense path; ``check=False`` skips that read (the caller inspects ``topk_status()`` later -- pipelined
-        callers and the device-timed benchmark loop).  ``fused=False`` forces the dense path."""
+        callers and the device-timed benchmark loop).  ``fused=False`` forces the dense path.
+
+        ``filt`` (``filters.RankFilter`` of the B rows): only the eligible items are ranked, excluded (row, item) pairs
+        are never returned, and rows with fewer than k returnable items end in (-1, -inf) padding.  Each shard ranks the
+        compact copy of its eligible rows (``_compact``) through the same paths, chosen by the number of eligible items;
+        a shard whose items are all eligible, with no exclusions, runs the unfiltered path."""
         kl = min(k, self.Vloc)
-        # results land in a ring of four preallocated buffers (no allocation in the query loop); a result stays valid
-        # for the next three topk calls
-        if self._topk_out is None or self._topk_out[0][0].shape[0] < B or self._topk_out[0][0].shape[1] != kl:
-            self._topk_out = [(torch.empty(max(B, 1), kl, dtype=torch.int32, device=self.dev),
-                               torch.empty(max(B, 1), kl, dtype=torch.float32, device=self.dev)) for _ in range(4)]
-            self._topk_i = 0
-        self._topk_i = (self._topk_i + 1) % 4
-        idx, val = self._topk_out[self._topk_i][0][:B], self._topk_out[self._topk_i][1][:B]
+        if _out is not None:        # a filtered call's shard ranked unfiltered: into that call's result buffers
+            idx, val = _out
+        else:
+            # results land in a ring of four preallocated buffers (no allocation in the query loop); a result stays
+            # valid for the next three topk calls
+            if self._topk_out is None or self._topk_out[0][0].shape[0] < B or self._topk_out[0][0].shape[1] != kl:
+                self._topk_out = [(torch.empty(max(B, 1), kl, dtype=torch.int32, device=self.dev),
+                                   torch.empty(max(B, 1), kl, dtype=torch.float32, device=self.dev))
+                                  for _ in range(4)]
+                self._topk_i = 0
+            self._topk_i = (self._topk_i + 1) % 4
+            idx, val = self._topk_out[self._topk_i][0][:B], self._topk_out[self._topk_i][1][:B]
+        if filt is not None:
+            ids = filt.shard_ids(self.V, self.rank, self.world)
+            excl = filt.exclude if filt.exclude is not None and filt.exclude.nnz else None   # rows without any
+            if ids is not None or excl is not None:
+                self._topk_filtered(B, kl, idx, val, scratch, mask_known, fused, check, ids, excl)
+            else:       # every item of this shard eligible, no exclusions: the unfiltered shard ranking
+                self.topk(B, kl, scratch=scratch, mask_known=mask_known, fused=fused, check=check, _out=(idx, val))
+            if self.world == 1:
+                return idx, val
+            oi, ov = self._merge_shards(B, k, idx, val, pad=-float("inf"))
+            ov.masked_fill_(oi < 0, -float("inf"))
+            return oi, ov
         impl = self.impl_for_scores()
         lib = N.load()
         mode, need = None, 0
@@ -1136,11 +1171,148 @@ class AAEEngine(object):
             call("aae_masked_topk", ptr(scratch), scratch.stride(0), B, self.Vloc, self.v_begin,
                  ptr(self.indptr) if mask_known else None, ptr(self.indices) if mask_known else None, kl, ptr(idx),
                  ptr(val), None, self._stream())
-        if self.world == 1:
+        if _out is not None or self.world == 1:
             return idx, val
         return self._merge_shards(B, k, idx, val)
 
-    def _merge_shards(self, B, k, idx, val):
+    def _compact(self, ids):
+        """Compact copy of this shard's eligible rows of the output layer: Wd3c [A,H] / bd3c [A] for the ascending
+        global ids ``ids`` (int32 numpy), with the device id table.  Cached: rebuilt when the eligible set or the
+        weights change (the padded Wp of the compact copy follows it lazily, ``_compact_padded``)."""
+        c = self._cmp
+        if c is not None and c["ver"] == self._wver and np.array_equal(c["ids_host"], ids):
+            return c
+        A = int(ids.size)
+        if c is None or c["cap"] < A:
+            cap = max(A, 1)
+            self._cmp = c = None    # free the old copy before the new one is allocated
+            c = dict(cap=cap, Wd3c=torch.empty(cap, self.H, dtype=torch.float32, device=self.dev),
+                     bd3c=torch.empty(cap, dtype=torch.float32, device=self.dev),
+                     ids=torch.empty(cap, dtype=torch.int32, device=self.dev), wp=None)
+        c.update(A=A, ids_host=ids.copy(), ver=self._wver, wp_ok=False)
+        if A:
+            c["ids"][:A].copy_(torch.from_numpy(ids))
+            call("aae_gather_item_rows", ptr(self.Wd3), ptr(self.bd3), self.H, self.Vloc, self.v_begin, ptr(c["ids"]), A,
+                 ptr(c["Wd3c"]), ptr(c["bd3c"]), ptr(self._n_bad), self._stream())
+            bad = int(self._n_bad.item())       # once per rebuild of the copy
+            if bad:
+                self._cmp = None
+                raise ValueError("%d of %d eligible ids are outside this shard's items [%d, %d) or not ascending"
+                                 % (bad, A, self.v_begin, self.v_end))
+        self._cmp = c
+        return c
+
+    def _compact_padded(self, c):
+        """``_padded_weights`` of the compact copy: Wp [A,104] and its largest row norm, so that the TF32 margin of the
+        v2 filter is that of exactly the rows being ranked."""
+        n = int(N.load().aae_pad_weights_floats(c["A"], self.H))
+        if c["wp"] is None or c["wp"].numel() < n:
+            c["wp"] = torch.empty(n, dtype=torch.float32, device=self.dev)
+            c["wp_ok"] = False
+        wmax = c["wp"][n - 64:]
+        if not c["wp_ok"]:
+            call("aae_pad_weights", ptr(c["Wd3c"]), ptr(c["bd3c"]), c["A"], self.H, ptr(c["wp"]), ptr(wmax),
+                 self._stream())
+            c["wp_ok"] = True
+        return c["wp"], wmax
+
+    def _upload_exclusions(self, X):
+        """Exclusion CSR of the batch (scipy, B rows) -> device (indptr, indices): one H2D copy from pinned staging,
+        both buffers grown geometrically (no allocation per batch)."""
+        B, nnz = X.shape[0], X.nnz
+        n = B + 1 + nnz
+        st = self._xstage
+        if st is None or st["cap"] < n:
+            cap = n if st is None else max(n, int(1.5 * st["cap"]))
+            if st is not None and st["ev"] is not None:
+                st["ev"].synchronize()
+            st = self._xstage = dict(cap=cap, pin=torch.empty(cap, dtype=torch.int32).pin_memory(),
+                                     dev=torch.empty(cap, dtype=torch.int32, device=self.dev), ev=None)
+        if st["ev"] is not None:
+            st["ev"].synchronize()      # the previous batch's copy has left the pinned buffer
+        host = st["pin"].numpy()
+        host[: B + 1] = X.indptr
+        host[B + 1: n] = X.indices
+        st["dev"][:n].copy_(st["pin"][:n], non_blocking=True)
+        ev = torch.cuda.Event()
+        ev.record(torch.cuda.current_stream(self.dev))
+        st["ev"] = ev
+        return st["dev"][: B + 1], st["dev"][B + 1: n]
+
+    def _topk_filtered(self, B, kl, idx, val, scratch, mask_known, fused, check, ids, exclude):
+        """Local ranking of one shard under a filter (see ``topk``): ``ids`` = the shard's eligible global ids (None:
+        all of them), ``exclude`` = the batch's exclusion CSR (None: none).  Same path choice as the unfiltered call,
+        on the number of eligible items A: fused v2 / v1 when A is inside their envelope (A >= 32768), else the dense
+        scores of the A columns + aae_masked_topk_filtered; A = 0 gives an all-padding list without a launch of the
+        ranking."""
+        # first, on every path: on item shards predict_h2 is a collective (the h1pre exchange), so a shard without
+        # eligible items must still take part in it
+        self.predict_h2(B)
+        if ids is not None and ids.size == 0:
+            idx.fill_(-1)
+            val.fill_(-float("inf"))
+            self.topk_mode = "empty"
+            return
+        if ids is None:
+            W, b, n, vb, ids_dev = self.Wd3, self.bd3, self.Vloc, self.v_begin, None
+        else:
+            c = self._compact(ids)
+            W, b, n, vb, ids_dev = c["Wd3c"], c["bd3c"], c["A"], 0, c["ids"]
+        xp, xi = self._upload_exclusions(exclude) if exclude is not None else (None, None)
+        filt = N.AaeRankFilter(ptr(ids_dev), ptr(xp), ptr(xi))
+        ip = ptr(self.indptr) if mask_known else None
+        ii = ptr(self.indices) if mask_known else None
+        impl = self.impl_for_scores()
+        lib = N.load()
+        mode, need = None, 0
+        want = os.environ.get("AAE_B200_TOPK", "")
+        if fused is not False and impl in (1, 2) and want != "dense":
+            if impl == 1 and want != "v1":
+                need = int(lib.aae_predict_topk2_work_bytes(B, n, kl, self.H))
+                mode = "v2" if need > 0 else None
+            if mode is None:
+                need = int(lib.aae_predict_topk_work_bytes(B, n, kl))
+                mode = "v1" if need > 0 else None
+        done = False
+        if mode is not None:
+            if self._topk_work is None or self._topk_work.numel() < need:
+                self._topk_work = torch.empty(need, dtype=torch.uint8, device=self.dev)
+            if mode == "v2":
+                wp, wmax = self._padded_weights() if ids is None else self._compact_padded(c)
+                call("aae_predict_topk2_filtered", ptr(self.h2), B, self.H, ptr(W), ptr(b), ptr(wp), ptr(wmax), n, vb,
+                     ip, ii, kl, ptr(self._topk_work), need, ptr(idx), ptr(val), ptr(self._n_bad), self._stream(),
+                     C.byref(filt))
+            else:
+                call("aae_predict_topk_filtered", ptr(self.h2), B, self.H, ptr(W), ptr(b), n, vb, ip, ii, kl, impl,
+                     ptr(self._topk_work), need, ptr(idx), ptr(val), ptr(self._n_bad), self._stream(), C.byref(filt))
+            self.topk_mode = mode
+            if check:
+                done = int(self._n_bad.item()) == 0
+                self.topk_fallbacks += 0 if done else 1
+            else:
+                done = True
+        if not done:
+            self.topk_mode = "dense"
+            if scratch is None or scratch.shape[0] < B or scratch.shape[1] < n:
+                scratch = torch.empty(B, n, dtype=torch.float32, device=self.dev)
+            call("aae_dec_out_scores", ptr(self.h2), B, self.H, ptr(W), ptr(b), n, 0, ptr(scratch), scratch.stride(0),
+                 impl, self._stream())
+            call("aae_masked_topk_filtered", ptr(scratch), scratch.stride(0), B, n, vb, ip, ii, kl, ptr(idx), ptr(val),
+                 None, self._stream(), C.byref(filt))
+
+    @_on_device
+    def compact_scores(self, B, ids):
+        """Logits of the batch in the device buffers for the eligible items ``ids`` only (ascending global ids, world
+        1): ([B, A] scores, device id table) -- the full-ranking path under a candidate filter."""
+        c = self._compact(ids)
+        out = torch.empty(B, max(c["A"], 1), dtype=torch.float32, device=self.dev)
+        if c["A"]:
+            self.predict_h2(B)
+            call("aae_dec_out_scores", ptr(self.h2), B, self.H, ptr(c["Wd3c"]), ptr(c["bd3c"]), c["A"], 0, ptr(out),
+                 out.stride(0), self.impl_for_scores(), self._stream())
+        return out[:, : c["A"]], c["ids"][: c["A"]]
+
+    def _merge_shards(self, B, k, idx, val, pad=-3.0e38):
         """Item shards -> global top-k: all-gather of the [B, kpad] per-shard lists into preallocated [world, B, kpad]
         buffers, then one merge kernel that reads that layout directly (no torch repacking in the query loop)."""
         import torch.distributed as dist
@@ -1162,6 +1334,9 @@ class AAEEngine(object):
             pv, pi = val.contiguous(), idx.contiguous()
         else:                                   # a last shard smaller than k: pad its list
             mb["pv"][:, :kl].copy_(val)
+            if mb.get("pad", -3.0e38) != pad:       # filtered calls pad with -inf
+                mb["pv"][:, kl:].fill_(pad)
+                mb["pad"] = pad
             mb["pi"][:, :kl].copy_(idx)
             pv, pi = mb["pv"], mb["pi"]
         dist.all_gather_into_tensor(mb["gv"], pv, group=self.group)

@@ -116,10 +116,11 @@ class VAE(AutoEncoder):
             out[start:end] = dev[:B].cpu().numpy()
         return out
 
-    def predict_topk(self, X, k, condition_data=None, mask_known=True, return_scores=False, shard="items"):
+    def predict_topk(self, X, k, condition_data=None, mask_known=True, return_scores=False, shard="items",
+                     items=None, exclude=None):
         self.engine.eval_injected = False          # ranking batches differ from the reference's: native noise
         return super().predict_topk(X, k, condition_data=condition_data, mask_known=mask_known,
-                                    return_scores=return_scores, shard=shard)
+                                    return_scores=return_scores, shard=shard, items=items, exclude=exclude)
 
 
 class VAERecommender(Recommender):
@@ -158,7 +159,7 @@ class VAERecommender(Recommender):
         X = test_set.tocsr()
         return self.model.predict(X, condition_data=self._condition_data(test_set, fit=False))
 
-    def predict_topk(self, test_set, k, mask_known=True):
+    def predict_topk(self, test_set, k, mask_known=True, items=None, exclude=None):
         X = test_set.tocsr()
         return self.model.predict_topk(X, k, condition_data=self._condition_data(test_set, fit=False),
-                                       mask_known=mask_known)
+                                       mask_known=mask_known, items=items, exclude=exclude)

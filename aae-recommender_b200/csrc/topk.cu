@@ -46,6 +46,72 @@ __global__ void mask_known_kernel(float* __restrict__ scores, int64_t lds, int B
   }
 }
 
+// Candidate filter of a ranking call (aae_rank_filter): the columns are the ascending global ids ids[0..n) (NULL:
+// v_begin + column), and excluded (row, id) pairs come as a CSR with sorted rows (NULL: none).
+struct RankFilt {
+  const int32_t* ids; const int32_t* xp; const int32_t* xi;
+};
+// true iff global id g is in CSR row `row` (sorted columns)
+__device__ __forceinline__ bool csr_has(const int32_t* __restrict__ indptr, const int32_t* __restrict__ indices, int row,
+                                        int g) {
+  int lo = indptr[row], hi = indptr[row + 1];
+  const int end = hi;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(indices + mid) < g) lo = mid + 1; else hi = mid;
+  }
+  return lo < end && __ldg(indices + lo) == g;
+}
+// column of global id g, or -1 when g is not a column
+__device__ __forceinline__ int col_of(const int32_t* __restrict__ ids, int n, int v_begin, int g) {
+  if (!ids) return (g >= v_begin && g - v_begin < n) ? g - v_begin : -1;
+  int lo = 0, hi = n;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(ids + mid) < g) lo = mid + 1; else hi = mid;
+  }
+  return (lo < n && __ldg(ids + lo) == g) ? lo : -1;
+}
+// mask_known_kernel on a filtered column set: scores[row, col_of(id)] = fill for every CSR entry whose id is a column
+// (fill = -FLT_MAX for the known items, -INFINITY for the exclusions)
+__global__ void mask_cols_kernel(float* __restrict__ scores, int64_t lds, int B, int n, int v_begin,
+                                 const int32_t* __restrict__ ids, const int32_t* __restrict__ indptr,
+                                 const int32_t* __restrict__ indices, float fill) {
+  const int nnz = indptr[B];
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += gridDim.x * blockDim.x) {
+    int lo = 0, hi = B;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (indptr[mid + 1] <= e) lo = mid + 1; else hi = mid;
+    }
+    const int c = col_of(ids, n, v_begin, indices[e]);
+    if (c >= 0) scores[(size_t)lo * lds + c] = fill;
+  }
+}
+// Compact copy of the eligible rows of an item shard: Wd3c[j,:] = Wd3[ids[j] - v_begin, :], bd3c[j] = bd3[...]; one warp
+// per row (float4 when H % 4 == 0).  An id outside the shard reads nothing (its row becomes zeros with bias -inf); ids
+// outside the shard or not above their predecessor are counted in *n_bad_ids.
+__global__ void gather_item_rows_kernel(const float* __restrict__ Wd3, const float* __restrict__ bd3, int H, int Vloc,
+                                        int v_begin, const int32_t* __restrict__ ids, int A, float* __restrict__ Wd3c,
+                                        float* __restrict__ bd3c, int32_t* __restrict__ n_bad_ids) {
+  const int lane = threadIdx.x & 31;
+  const int nw = (gridDim.x * blockDim.x) >> 5;
+  for (int j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < A; j += nw) {
+    const int r = ids[j] - v_begin;
+    const bool in = r >= 0 && r < Vloc;
+    if (lane == 0 && (!in || (j > 0 && ids[j - 1] >= ids[j]))) atomicAdd(n_bad_ids, 1);
+    float* dst = Wd3c + (size_t)j * H;
+    if ((H & 3) == 0) {
+      const float4* src = reinterpret_cast<const float4*>(Wd3 + (size_t)(in ? r : 0) * H);
+      for (int c = lane; c < (H >> 2); c += 32)
+        reinterpret_cast<float4*>(dst)[c] = in ? __ldg(src + c) : make_float4(0.f, 0.f, 0.f, 0.f);
+    } else {
+      for (int c = lane; c < H; c += 32) dst[c] = in ? __ldg(Wd3 + (size_t)r * H + c) : 0.f;
+    }
+    if (lane == 0) bd3c[j] = in ? __ldg(bd3 + r) : -INFINITY;
+  }
+}
+
 // descending bitonic sort of n (power of two) 64-bit composites in shared memory
 __device__ void bitonic_desc(unsigned long long* a, int n) {
   for (int size = 2; size <= n; size <<= 1) {
@@ -107,12 +173,16 @@ __device__ int block_count_ge(const float* __restrict__ row, int n, uint32_t thr
 }
 
 // idx_map == nullptr: candidates are row positions (+ idx_offset); else idx_out = idx_map[row, pos]
+// FILT: the id found that way is a column of a filtered set: emitted as ids[id] (ids NULL: as is); entries scored
+// -INFINITY (excluded) and the padding of rows shorter than k are emitted as (-1, -INFINITY)
+template <bool FILT>
 __global__ void __launch_bounds__(TK_THREADS, 1) row_topk_kernel(const float* __restrict__ scores, int64_t lds, int n,
                                                                  int k, int idx_offset,
                                                                  const int32_t* __restrict__ idx_map,
                                                                  const int32_t* __restrict__ n_valid,
                                                                  int skip_upto, int32_t* __restrict__ idx_out,
-                                                                 float* __restrict__ val_out) {
+                                                                 float* __restrict__ val_out,
+                                                                 const int32_t* __restrict__ ids) {
   extern __shared__ __align__(16) unsigned char sm_raw[];
   unsigned long long* buf = reinterpret_cast<unsigned long long*>(sm_raw);          // [TK_CAP]
   uint32_t* samp = reinterpret_cast<uint32_t*>(buf + TK_CAP);                       // [TK_SAMPLE] (as u64 pairs)
@@ -186,12 +256,13 @@ __global__ void __launch_bounds__(TK_THREADS, 1) row_topk_kernel(const float* __
   bitonic_desc(buf, npow);
   for (int i = threadIdx.x; i < k; i += blockDim.x) {
     int32_t id = -1;
-    float val = -FLT_MAX;
+    float val = FILT ? -INFINITY : -FLT_MAX;
     if (i < kk) {
       unsigned long long c = buf[i];
       uint32_t pos = 0xFFFFFFFFu - (uint32_t)(c & 0xFFFFFFFFull);
       id = direct_ids ? (int32_t)pos : (idx_map ? idx_map[(size_t)rowi * lds + pos] : (int32_t)pos + idx_offset);
       val = key2f((uint32_t)(c >> 32));
+      if (FILT) id = (val == -INFINITY || id < 0) ? -1 : (ids ? ids[id] : id);
     }
     idx_out[(size_t)rowi * k + i] = id;
     if (val_out) val_out[(size_t)rowi * k + i] = val;
@@ -210,8 +281,11 @@ __global__ void __launch_bounds__(TK_THREADS, 1) row_topk_kernel(const float* __
 struct RescoreArgs {
   const float* h2; const float* Wd3; const float* bd3; int H; int v_begin;
 };
+// FILT: the candidate ids are columns of a filtered set (global id f.ids[id], or id itself when f.ids is NULL): known
+// items are looked up by global id, excluded candidates are dropped (value -INFINITY, not counted as returnable); the
+// ids stay columns (the final sort translates them), so that re-scoring reads compact row `id`.
 constexpr int FIN_THREADS = 256;
-template <bool RESCORE>
+template <bool RESCORE, bool FILT>
 __global__ void __launch_bounds__(FIN_THREADS) cand_finish_kernel(const float* __restrict__ cand_val,
                                                                   const int32_t* __restrict__ cand_idx,
                                                                   const int32_t* __restrict__ cnt, int nsub, int cap_sub,
@@ -219,7 +293,7 @@ __global__ void __launch_bounds__(FIN_THREADS) cand_finish_kernel(const float* _
                                                                   int cap_out, int32_t* __restrict__ tot, int B, int k,
                                                                   const int32_t* __restrict__ indptr,
                                                                   const int32_t* __restrict__ indices, int32_t* n_bad,
-                                                                  RescoreArgs ra) {
+                                                                  RescoreArgs ra, RankFilt f) {
   extern __shared__ int off_s[];                 // [nsub + 1] exclusive prefix of the sub-list counts (+ h2 row if RESCORE)
   __shared__ int warp_s[FIN_THREADS / 32];
   __shared__ int valid_s, over_s;
@@ -270,12 +344,14 @@ __global__ void __launch_bounds__(FIN_THREADS) cand_finish_kernel(const float* _
         const size_t src = ((size_t)row * nsub + sidx) * cap_sub + sl;
         const int id = cand_idx[src];
         float v = RESCORE ? 0.f : cand_val[src];
+        const int g = (FILT && f.ids) ? __ldg(f.ids + id) : id;
         int lo = p0, hi = p1;
         while (lo < hi) {
           const int mid = (lo + hi) >> 1;
-          if (__ldg(indices + mid) < id) lo = mid + 1; else hi = mid;
+          if (__ldg(indices + mid) < g) lo = mid + 1; else hi = mid;
         }
-        if (lo < p1 && __ldg(indices + lo) == id) v = -FLT_MAX;
+        if (FILT && f.xp && csr_has(f.xp, f.xi, row, g)) v = -INFINITY;
+        else if (lo < p1 && __ldg(indices + lo) == g) v = -FLT_MAX;
         else ++valid;
         out_val[(size_t)row * cap_out + o0 + sl] = v;
         out_idx[(size_t)row * cap_out + o0 + sl] = id;
@@ -300,7 +376,8 @@ __global__ void __launch_bounds__(FIN_THREADS) cand_finish_kernel(const float* _
       for (int c0 = warp * 4; c0 < total; c0 += (FIN_THREADS / 32) * 4) {
         const int c = c0 + sub;
         const size_t o = (size_t)row * cap_out + c;
-        const bool live = c < total && out_val[o] != -FLT_MAX;       // -FLT_MAX: a known item, stays at the bottom
+        // -FLT_MAX: a known item, stays at the bottom; -INFINITY: an excluded one
+        const bool live = c < total && out_val[o] != -FLT_MAX && (!FILT || out_val[o] != -INFINITY);
         float acc = 0.f;
         int item = 0;
         if (live) {
@@ -361,12 +438,15 @@ __global__ void check_kth_kernel(const float* __restrict__ val, int k, const flo
 // 256 threads and 16 KB of shared memory per row instead of 1024 threads and 96 KB, so that eight rows are sorted per
 // SM at a time.  Rows with more than CS_CAP live candidates are left to row_topk_kernel (skip_upto = CS_CAP there).
 // Composites carry the item id: descending score, ties by lower id -- the same order as row_topk_kernel.
+// FILT: ids are translated and excluded / padding entries emitted as in row_topk_kernel<true>.
 constexpr int CS_THREADS = 256, CS_CAP = 2048;
+template <bool FILT>
 __global__ void __launch_bounds__(CS_THREADS) cand_sort_small_kernel(const float* __restrict__ val,
                                                                      const int32_t* __restrict__ idx, int64_t lds,
                                                                      const int32_t* __restrict__ n_valid, int k,
                                                                      int32_t* __restrict__ idx_out,
-                                                                     float* __restrict__ val_out) {
+                                                                     float* __restrict__ val_out,
+                                                                     const int32_t* __restrict__ ids) {
   __shared__ unsigned long long buf[CS_CAP];
   const int rowi = blockIdx.x;
   const int n = n_valid[rowi];
@@ -379,11 +459,12 @@ __global__ void __launch_bounds__(CS_THREADS) cand_sort_small_kernel(const float
   const int kk = min(k, n);
   for (int i = threadIdx.x; i < k; i += CS_THREADS) {
     int32_t id = -1;
-    float v = -FLT_MAX;
+    float v = FILT ? -INFINITY : -FLT_MAX;
     if (i < kk) {
       const unsigned long long c = buf[i];
       id = (int32_t)(0xFFFFFFFFu - (uint32_t)(c & 0xFFFFFFFFull));
       v = key2f((uint32_t)(c >> 32));
+      if (FILT) id = v == -INFINITY ? -1 : (ids ? ids[id] : id);
     }
     idx_out[(size_t)rowi * k + i] = id;
     if (val_out) val_out[(size_t)rowi * k + i] = v;
@@ -565,22 +646,38 @@ __global__ void __launch_bounds__(RC_THREADS) rank_count_kernel(const float* __r
 
 using namespace aae;
 
-extern "C" {
-
-
+template <bool FILT = false>
 static int launch_row_topk(const float* scores, int64_t lds, int B, int n, int k, int idx_offset,
                            const int32_t* idx_map, int32_t* idx_out, float* val_out, cudaStream_t s,
-                           const int32_t* n_valid = nullptr, int skip_upto = -1) {
+                           const int32_t* n_valid = nullptr, int skip_upto = -1, const int32_t* ids = nullptr) {
   size_t smem = sizeof(unsigned long long) * (TK_CAP + TK_SAMPLE);
-  cudaError_t e = cudaFuncSetAttribute(row_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(row_topk_kernel<FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) {
     set_error("row_topk: %s", cudaGetErrorString(e));
     return AAE_E_CUDA;
   }
-  row_topk_kernel<<<B, TK_THREADS, smem, s>>>(scores, lds, n, k, idx_offset, idx_map, n_valid, skip_upto, idx_out,
-                                              val_out);
+  row_topk_kernel<FILT><<<B, TK_THREADS, smem, s>>>(scores, lds, n, k, idx_offset, idx_map, n_valid, skip_upto, idx_out,
+                                                    val_out, ids);
   return check_launch("row_topk");
 }
+
+static bool filter_active(const aae_rank_filter* f) { return f && (f->item_ids || f->excl_indptr); }
+
+// Arguments every *_filtered entry point checks: the exclusion CSR comes whole, and a column table implies v_begin 0
+// (the ranked matrix is the compact copy of aae_gather_item_rows).
+static int check_filter(const aae_rank_filter* f, int v_begin, const char* fn) {
+  if ((f->excl_indptr == nullptr) != (f->excl_indices == nullptr)) {
+    set_error("%s: excl_indptr and excl_indices go together", fn);
+    return AAE_E_ARG;
+  }
+  if (f->item_ids && v_begin != 0) {
+    set_error("%s: a column table (item_ids) ranks a compact matrix: v_begin must be 0", fn);
+    return AAE_E_ARG;
+  }
+  return AAE_OK;
+}
+
+extern "C" {
 
 int aae_masked_topk(float* scores, int64_t lds, int B, int Vloc, int v_begin, const int32_t* indptr,
                     const int32_t* indices, int k, int32_t* idx_out, float* val_out, void* work, void* stream) {
@@ -594,6 +691,46 @@ int aae_masked_topk(float* scores, int64_t lds, int B, int Vloc, int v_begin, co
     if (rc) return rc;
   }
   return launch_row_topk(scores, lds, B, Vloc, k, v_begin, nullptr, idx_out, val_out, as_stream(stream));
+}
+
+int aae_masked_topk_filtered(float* scores, int64_t lds, int B, int Vloc, int v_begin, const int32_t* indptr,
+                             const int32_t* indices, int k, int32_t* idx_out, float* val_out, void* work, void* stream,
+                             const aae_rank_filter* filt) {
+  if (!filter_active(filt))
+    return aae_masked_topk(scores, lds, B, Vloc, v_begin, indptr, indices, k, idx_out, val_out, work, stream);
+  AAE_REQUIRE(scores && idx_out, "null pointer");
+  AAE_REQUIRE(k > 0 && k <= TK_CAP / 2, "k outside the supported envelope (1..4096)");
+  AAE_REQUIRE(B > 0 && Vloc > 0, "bad size");
+  int rc = check_filter(filt, v_begin, __func__);
+  if (rc) return rc;
+  cudaStream_t s = as_stream(stream);
+  const int grid = std::min(4 * sm_count(), std::max(1, cdiv((int64_t)B * 32, 256)));
+  if (indptr && indices) {
+    mask_cols_kernel<<<grid, 256, 0, s>>>(scores, lds, B, Vloc, v_begin, filt->item_ids, indptr, indices, -FLT_MAX);
+    rc = check_launch("mask_cols(known)");
+    if (rc) return rc;
+  }
+  if (filt->excl_indptr) {
+    mask_cols_kernel<<<grid, 256, 0, s>>>(scores, lds, B, Vloc, v_begin, filt->item_ids, filt->excl_indptr,
+                                          filt->excl_indices, -INFINITY);
+    rc = check_launch("mask_cols(exclude)");
+    if (rc) return rc;
+  }
+  return launch_row_topk<true>(scores, lds, B, Vloc, k, v_begin, nullptr, idx_out, val_out, s, nullptr, -1,
+                               filt->item_ids);
+}
+
+int aae_gather_item_rows(const float* Wd3, const float* bd3, int H, int Vloc, int v_begin, const int32_t* item_ids,
+                         int A, float* Wd3c, float* bd3c, int32_t* n_bad, void* stream) {
+  AAE_REQUIRE(Wd3 && bd3 && item_ids && Wd3c && bd3c && n_bad, "null pointer");
+  AAE_REQUIRE(H > 0 && Vloc > 0 && A > 0, "bad size");
+  AAE_REQUIRE((H & 3) != 0 || ((reinterpret_cast<uintptr_t>(Wd3) | reinterpret_cast<uintptr_t>(Wd3c)) & 15) == 0,
+              "Wd3 and Wd3c must be 16-byte aligned");
+  cudaStream_t s = as_stream(stream);
+  cudaMemsetAsync(n_bad, 0, sizeof(int32_t), s);
+  gather_item_rows_kernel<<<std::min(8 * sm_count(), std::max(1, cdiv((int64_t)A * 32, 256))), 256, 0, s>>>(
+      Wd3, bd3, H, Vloc, v_begin, item_ids, A, Wd3c, bd3c, n_bad);
+  return check_launch("gather_item_rows");
 }
 
 int aae_rank_counts(float* scores, int64_t lds, int B, int Vloc, int v_begin, const int32_t* indptr,
@@ -628,9 +765,10 @@ int64_t aae_predict_topk_work_bytes(int B, int Vloc, int k) {
                    2 * al256((size_t)B * p.cap * 4));
 }
 
-int aae_predict_topk(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int v_begin,
-                     const int32_t* indptr, const int32_t* indices, int k, int impl, void* work, int64_t work_bytes,
-                     int32_t* idx_out, float* val_out, int32_t* n_bad, void* stream) {
+static int predict_topk_impl(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int v_begin,
+                             const int32_t* indptr, const int32_t* indices, int k, int impl, void* work,
+                             int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad, void* stream,
+                             const aae_rank_filter* filt) {
   AAE_REQUIRE(h2 && Wd3 && bd3 && idx_out && n_bad && work, "null pointer");
   AAE_REQUIRE(B > 0 && H > 0 && Vloc > 0 && k > 0, "bad size");
   AAE_REQUIRE((indptr == nullptr) == (indices == nullptr), "indptr and indices go together");
@@ -675,15 +813,50 @@ int aae_predict_topk(const float* h2, int B, int H, const float* Wd3, const floa
                          kth_fast ? thr_val : thr_val + (p.J - 1), kth_fast ? 1 : p.J, cnt, sub_val, sub_idx, p.cap_sub,
                          split, s);
   if (rc) return rc;
-  cand_finish_kernel<false><<<std::min(B, 8 * sm_count()), FIN_THREADS, (p.nsub + 1) * sizeof(int), s>>>(
-      sub_val, sub_idx, cnt, p.nsub, p.cap_sub, cand_val, cand_idx, p.cap, tot, B, std::min(k, Vloc), indptr, indices,
-      n_bad, RescoreArgs{nullptr, nullptr, nullptr, 0, 0});
+  const int fin_grid = std::min(B, 8 * sm_count());
+  const size_t fin_smem = (p.nsub + 1) * sizeof(int);
+  const RescoreArgs ra{nullptr, nullptr, nullptr, 0, 0};
+  if (filt) {
+    const RankFilt rf{filt->item_ids, filt->excl_indptr, filt->excl_indices};
+    cand_finish_kernel<false, true><<<fin_grid, FIN_THREADS, fin_smem, s>>>(
+        sub_val, sub_idx, cnt, p.nsub, p.cap_sub, cand_val, cand_idx, p.cap, tot, B, std::min(k, Vloc), indptr, indices,
+        n_bad, ra, rf);
+  } else {
+    cand_finish_kernel<false, false><<<fin_grid, FIN_THREADS, fin_smem, s>>>(
+        sub_val, sub_idx, cnt, p.nsub, p.cap_sub, cand_val, cand_idx, p.cap, tot, B, std::min(k, Vloc), indptr, indices,
+        n_bad, ra, RankFilt{nullptr, nullptr, nullptr});
+  }
   rc = check_launch("cand_finish");
   if (rc) return rc;
-  cand_sort_small_kernel<<<B, CS_THREADS, 0, s>>>(cand_val, cand_idx, p.cap, tot, k, idx_out, val_out);
+  if (filt) cand_sort_small_kernel<true><<<B, CS_THREADS, 0, s>>>(cand_val, cand_idx, p.cap, tot, k, idx_out, val_out,
+                                                                  filt->item_ids);
+  else cand_sort_small_kernel<false><<<B, CS_THREADS, 0, s>>>(cand_val, cand_idx, p.cap, tot, k, idx_out, val_out,
+                                                              nullptr);
   rc = check_launch("cand_sort_small");
   if (rc) return rc;
+  if (filt)
+    return launch_row_topk<true>(cand_val, p.cap, B, p.cap, k, 0, cand_idx, idx_out, val_out, s, tot, CS_CAP,
+                                 filt->item_ids);
   return launch_row_topk(cand_val, p.cap, B, p.cap, k, 0, cand_idx, idx_out, val_out, s, tot, CS_CAP);
+}
+
+int aae_predict_topk(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int v_begin,
+                     const int32_t* indptr, const int32_t* indices, int k, int impl, void* work, int64_t work_bytes,
+                     int32_t* idx_out, float* val_out, int32_t* n_bad, void* stream) {
+  return predict_topk_impl(h2, B, H, Wd3, bd3, Vloc, v_begin, indptr, indices, k, impl, work, work_bytes, idx_out,
+                           val_out, n_bad, stream, nullptr);
+}
+
+int aae_predict_topk_filtered(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int v_begin,
+                              const int32_t* indptr, const int32_t* indices, int k, int impl, void* work,
+                              int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad, void* stream,
+                              const aae_rank_filter* filt) {
+  if (filter_active(filt)) {
+    const int rc = check_filter(filt, v_begin, __func__);
+    if (rc) return rc;
+  }
+  return predict_topk_impl(h2, B, H, Wd3, bd3, Vloc, v_begin, indptr, indices, k, impl, work, work_bytes, idx_out,
+                           val_out, n_bad, stream, filter_active(filt) ? filt : nullptr);
 }
 
 int64_t aae_predict_topk2_work_bytes(int B, int Vloc, int k, int H) {
@@ -695,9 +868,10 @@ int64_t aae_predict_topk2_work_bytes(int B, int Vloc, int k, int H) {
                    2 * al256((size_t)B * p.cap * 4) + al256((size_t)B * k * 4));
 }
 
-int aae_predict_topk2(const float* h2, int B, int H, const float* Wd3, const float* bd3, const float* Wp,
-                      const float* wmax, int Vloc, int v_begin, const int32_t* indptr, const int32_t* indices, int k,
-                      void* work, int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad, void* stream) {
+static int predict_topk2_impl(const float* h2, int B, int H, const float* Wd3, const float* bd3, const float* Wp,
+                              const float* wmax, int Vloc, int v_begin, const int32_t* indptr, const int32_t* indices,
+                              int k, void* work, int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad,
+                              void* stream, const aae_rank_filter* filt) {
   AAE_REQUIRE(h2 && Wd3 && bd3 && Wp && wmax && idx_out && n_bad && work, "null pointer");
   AAE_REQUIRE(B > 0 && H > 0 && Vloc > 0 && k > 0, "bad size");
   AAE_REQUIRE((indptr == nullptr) == (indices == nullptr), "indptr and indices go together");
@@ -745,18 +919,50 @@ int aae_predict_topk2(const float* h2, int B, int H, const float* Wd3, const flo
   cudaMemsetAsync(n_bad, 0, 4, s);
   rc = dec_out_select2(h2, B, H, Wp, Vloc, v_begin, 1, p.n_tiles, 1, nullptr, 0, 0, tau_f, cnt, sub_idx, p.cap_sub, s);
   if (rc) return rc;
-  cand_finish_kernel<true><<<std::min(B, 8 * sm_count()), FIN_THREADS, ((p.nsub + 4) & ~3) * sizeof(int) + H * sizeof(float) + 16,
-                             s>>>(nullptr, sub_idx, cnt, p.nsub, p.cap_sub, cand_val, cand_idx, p.cap, tot, B, kk, indptr,
-                                  indices, n_bad, RescoreArgs{h2, Wd3, bd3, H, v_begin});
+  const int fin_grid = std::min(B, 8 * sm_count());
+  const size_t fin_smem = ((p.nsub + 4) & ~3) * sizeof(int) + H * sizeof(float) + 16;
+  const RescoreArgs ra{h2, Wd3, bd3, H, v_begin};
+  if (filt) {
+    const RankFilt rf{filt->item_ids, filt->excl_indptr, filt->excl_indices};
+    cand_finish_kernel<true, true><<<fin_grid, FIN_THREADS, fin_smem, s>>>(
+        nullptr, sub_idx, cnt, p.nsub, p.cap_sub, cand_val, cand_idx, p.cap, tot, B, kk, indptr, indices, n_bad, ra, rf);
+  } else {
+    cand_finish_kernel<true, false><<<fin_grid, FIN_THREADS, fin_smem, s>>>(
+        nullptr, sub_idx, cnt, p.nsub, p.cap_sub, cand_val, cand_idx, p.cap, tot, B, kk, indptr, indices, n_bad, ra,
+        RankFilt{nullptr, nullptr, nullptr});
+  }
   rc = check_launch("cand_finish(rescore)");
   if (rc) return rc;
-  cand_sort_small_kernel<<<B, CS_THREADS, 0, s>>>(cand_val, cand_idx, p.cap, tot, k, idx_out, vout);
+  if (filt) cand_sort_small_kernel<true><<<B, CS_THREADS, 0, s>>>(cand_val, cand_idx, p.cap, tot, k, idx_out, vout,
+                                                                  filt->item_ids);
+  else cand_sort_small_kernel<false><<<B, CS_THREADS, 0, s>>>(cand_val, cand_idx, p.cap, tot, k, idx_out, vout, nullptr);
   rc = check_launch("cand_sort_small");
   if (rc) return rc;
-  rc = launch_row_topk(cand_val, p.cap, B, p.cap, k, 0, cand_idx, idx_out, vout, s, tot, CS_CAP);
+  rc = filt ? launch_row_topk<true>(cand_val, p.cap, B, p.cap, k, 0, cand_idx, idx_out, vout, s, tot, CS_CAP,
+                                    filt->item_ids)
+            : launch_row_topk(cand_val, p.cap, B, p.cap, k, 0, cand_idx, idx_out, vout, s, tot, CS_CAP);
   if (rc) return rc;
   check_kth_kernel<<<cdiv(B, 256), 256, 0, s>>>(vout, k, thr, thr_stride, tot, B, n_bad);
   return check_launch("check_kth");
+}
+
+int aae_predict_topk2(const float* h2, int B, int H, const float* Wd3, const float* bd3, const float* Wp,
+                      const float* wmax, int Vloc, int v_begin, const int32_t* indptr, const int32_t* indices, int k,
+                      void* work, int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad, void* stream) {
+  return predict_topk2_impl(h2, B, H, Wd3, bd3, Wp, wmax, Vloc, v_begin, indptr, indices, k, work, work_bytes, idx_out,
+                            val_out, n_bad, stream, nullptr);
+}
+
+int aae_predict_topk2_filtered(const float* h2, int B, int H, const float* Wd3, const float* bd3, const float* Wp,
+                               const float* wmax, int Vloc, int v_begin, const int32_t* indptr, const int32_t* indices,
+                               int k, void* work, int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad,
+                               void* stream, const aae_rank_filter* filt) {
+  if (filter_active(filt)) {
+    const int rc = check_filter(filt, v_begin, __func__);
+    if (rc) return rc;
+  }
+  return predict_topk2_impl(h2, B, H, Wd3, bd3, Wp, wmax, Vloc, v_begin, indptr, indices, k, work, work_bytes, idx_out,
+                            val_out, n_bad, stream, filter_active(filt) ? filt : nullptr);
 }
 
 int aae_topk_merge_seg(const float* cand_val, const int32_t* cand_idx, int world, int B, int kpad, int k,

@@ -312,6 +312,45 @@ int aae_predict_topk2(const float* h2, int B, int H, const float* Wd3, const flo
                       const float* wmax, int Vloc, int v_begin, const int32_t* indptr, const int32_t* indices, int k,
                       void* work, int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad, void* stream);
 
+/* ---- candidate-restricted ranking (predict_topk(..., items=, exclude=)) -----------------------------------------
+ * Replaces ranking every item and filtering the list afterwards (which leaves rows short): the eligible items of a shard
+ * are gathered into a compact output layer [A, H] / [A] (aae_gather_item_rows) and the ranking entry points run on it
+ * with v_begin = 0, so that the GEMM work, the weight bytes and the TF32 error bound (aae_pad_weights on the compact
+ * copy) all follow the eligible set.  The filter tells the ranking which global id each compact column stands for and
+ * which (row, item) pairs must never be returned:
+ *   item_ids     [n_cols] global id of each column, strictly ascending; NULL: column c is item v_begin + c (with a table,
+ *                v_begin must be 0)
+ *   excl_indptr  [B+1] / excl_indices: per-row exclusions (global ids, sorted within each row); NULL: none
+ * Known items (indptr/indices, global ids) that are columns rank below every other item (-FLT_MAX) as in the unfiltered
+ * calls; excluded items and the padding of rows with fewer than k returnable items come out as (-1, -INFINITY).  Ties
+ * go to the lower item id.  A NULL filter, or one with both tables NULL, is exactly the unfiltered call.  The fused
+ * calls count rows with fewer than k returnable candidates in n_bad, like overflowing rows: the dense pair
+ * aae_dec_out_scores + aae_masked_topk_filtered then gives the exact, padded answer. */
+typedef struct {
+  const int32_t* item_ids;
+  const int32_t* excl_indptr;
+  const int32_t* excl_indices;
+} aae_rank_filter;
+/* Wd3c[j,:] = Wd3[item_ids[j] - v_begin, :], bd3c[j] = bd3[item_ids[j] - v_begin] for j < A (one warp per row; float4
+ * when H % 4 == 0, then Wd3 and Wd3c 16-byte aligned).  Checks the table: n_bad[0] (device) receives the number of
+ * ids that lie outside [v_begin, v_begin + Vloc) or are not above their predecessor; it must be 0 before the copy is
+ * used (a bad id's row is not read and is written as zeros with bias -INFINITY).  Replaces indexing the shard's
+ * output layer on the host. */
+int aae_gather_item_rows(const float* Wd3, const float* bd3, int H, int Vloc, int v_begin, const int32_t* item_ids,
+                         int A, float* Wd3c, float* bd3c, int32_t* n_bad, void* stream);
+/* aae_masked_topk / aae_predict_topk / aae_predict_topk2 on a filtered column set (Vloc = number of columns). */
+int aae_masked_topk_filtered(float* scores, int64_t lds, int B, int Vloc, int v_begin, const int32_t* indptr,
+                             const int32_t* indices, int k, int32_t* idx_out, float* val_out, void* work, void* stream,
+                             const aae_rank_filter* filt);
+int aae_predict_topk_filtered(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int v_begin,
+                              const int32_t* indptr, const int32_t* indices, int k, int impl, void* work,
+                              int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad, void* stream,
+                              const aae_rank_filter* filt);
+int aae_predict_topk2_filtered(const float* h2, int B, int H, const float* Wd3, const float* bd3, const float* Wp,
+                               const float* wmax, int Vloc, int v_begin, const int32_t* indptr, const int32_t* indices,
+                               int k, void* work, int64_t work_bytes, int32_t* idx_out, float* val_out, int32_t* n_bad,
+                               void* stream, const aae_rank_filter* filt);
+
 /* ---- GPU-side ranking metrics (SURVEY 8(f)-2) -----------------------------------------------------
  * Replaces the dense D2H + host argsort behind the harness' metrics (evaluation.py:70-164 RankingMetric / MRR /
  * MAP / P, evaluate 202-240 on remove_non_missing(predict(X), X)): for every held-out ("gold") item of every
