@@ -274,9 +274,11 @@ class AAEEngine(object):
         return 1 if ok else 0
 
     def impl_for_scores(self):
+        """Scores / fused v1 kernel: 1 = tcgen05 3xTF32 (n_hidden % 4 == 0, n_hidden <= 108: a [Wd3 | bd3] row of at
+        most 112 floats fits its operand tile), 0 = fp32 CUDA cores (any n_hidden up to 512)."""
         if self.impl >= 0:
             return self.impl
-        return 1 if (self.H % 4 == 0 and self.H <= 124) else 0
+        return 1 if (self.H % 4 == 0 and self.H <= 108) else 0
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.dev).cuda_stream)
@@ -1242,7 +1244,7 @@ class AAEEngine(object):
     def _topk_filtered(self, B, kl, idx, val, scratch, mask_known, fused, check, ids, exclude):
         """Local ranking of one shard under a filter (see ``topk``): ``ids`` = the shard's eligible global ids (None:
         all of them), ``exclude`` = the batch's exclusion CSR (None: none).  Same path choice as the unfiltered call,
-        on the number of eligible items A: fused v2 / v1 when A is inside their envelope (A >= 32768), else the dense
+        on the number of eligible items A: fused v2 / v1 when A is inside their envelope (A >= 32641), else the dense
         scores of the A columns + aae_masked_topk_filtered; A = 0 gives an all-padding list without a launch of the
         ranking."""
         # first, on every path: on item shards predict_h2 is a collective (the h1pre exchange), so a shard without

@@ -277,6 +277,13 @@ int dec_out_select_tc(const float* h2, int B, int H, const float* Wd3, const flo
                       int32_t* cand_idx, int cap, int split, cudaStream_t s) {
   if (!tc_supported(B, H, "dec_out_select")) return AAE_E_UNSUPPORTED;
   tc::Geom g = tc::make_geom(H);
+  // The loaders cover 4 * P_WCH 16-byte column groups of a W' row, and two stages of hi and lo operands of Kp = 112
+  // floats (229 KB) are what the shared memory holds: longer rows (n_hidden 112 .. 124) are not supported here.
+  if (g.Kp > 16 * tc::P_WCH) {
+    set_error("dec_out_select: n_hidden %d needs W' rows of %d floats, the tensor-core scores kernel holds %d "
+              "(n_hidden <= %d): use impl 0", H, g.Kp, 16 * tc::P_WCH, 16 * tc::P_WCH - 4);
+    return AAE_E_UNSUPPORTED;
+  }
   const size_t smem = 4 * (size_t)(tc::PN / 8) * g.wb_sbo + 256;
   auto kern = (split == 3) ? tc::dec_out_select_kernel<3> : tc::dec_out_select_kernel<1>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -553,7 +553,7 @@ static TopkPlan make_plan(int B, int Vloc, int k, bool v2 = false) {
   TopkPlan p;
   p.n_tiles = (Vloc + 127) / 128;
   p.n_samp = std::min(512, p.n_tiles / 8);
-  p.ok = p.n_samp >= 32 && k <= 1024;          // Vloc >= 32768; below that the dense path is as cheap
+  p.ok = p.n_samp >= 32 && k <= 1024;          // Vloc >= 32641 (256 tiles); below that the dense path is as cheap
   p.stride = p.ok ? p.n_tiles / p.n_samp : 1;
   p.S = p.n_samp * 128;
   p.T = std::max(1024, std::min(4096, 4 * (k + 256)));

@@ -245,7 +245,7 @@ int aae_masked_topk(float* scores, int64_t lds, int B, int Vloc, int v_begin, co
  * lists, (4) known items masked, candidates sorted, first k emitted (descending, ties by lower item id).
  * Exactness never depends on the estimate: n_bad[0] (device) counts rows whose list overflowed or held fewer than
  * k unknown items; if it is non-zero the caller must rank the batch through aae_dec_out_scores + aae_masked_topk.
- * Envelope: impl 1 (3xTF32) or 2 (TF32), Vloc >= 32768, k <= 1024; otherwise AAE_E_UNSUPPORTED.
+ * Envelope: impl 1 (3xTF32) or 2 (TF32), Vloc >= 32641 (256 tiles of 128 items), k <= 1024; otherwise AAE_E_UNSUPPORTED.
  * work: aae_predict_topk_work_bytes(B, Vloc, k) bytes of device scratch (0 = outside the envelope). */
 int64_t aae_predict_topk_work_bytes(int B, int Vloc, int k);
 int aae_predict_topk(const float* h2, int B, int H, const float* Wd3, const float* bd3, int Vloc, int v_begin,

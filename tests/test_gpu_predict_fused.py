@@ -31,7 +31,7 @@ def _oracle_logits(eng, X):
 @pytest.mark.parametrize("V,B,k", [(40000, 70, 100), (150001, 200, 20), (70000, 130, 500), (300000, 1100, 100)])
 def test_fused_topk_matches_oracle_and_dense_path(V, B, k, mode, monkeypatch):
     """mode v2: TMA-multicast single-pass TF32 filter + exact fp32 re-scoring of the survivors (aae_predict_topk2; a
-    cluster of 1, 2 or 8 row-chunk CTAs for these batch sizes); mode v1: the 3xTF32 filter (aae_predict_topk)."""
+    cluster of 1, 2 or 4 row-chunk CTAs for these batch sizes); mode v1: the 3xTF32 filter (aae_predict_topk)."""
     from aaerec_b200.synth import synth_sets
     from oracle import aae_oracle as O
     if mode == "v1":
