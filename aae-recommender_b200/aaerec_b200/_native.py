@@ -82,6 +82,7 @@ _SIGS = {
     "aae_topk_merge": (I, [P, P, I, I, I, P, P, P]),
     "aae_topk_merge_seg": (I, [P, P, I, I, I, I, P, P, P]),
     "aae_rank_counts": (I, [P, I64, I, I, I, P, P, P, P, I, P, I, P, P]),
+    "aae_rank_counts_filtered": (I, [P, I64, I, I, I, P, P, P, P, I, P, I, P, P, C.POINTER(AaeRankFilter)]),
     "aae_predict_topk_work_bytes": (I64, [I, I, I]),
     "aae_predict_topk": (I, [P, I, I, P, P, I, I, P, P, I, I, P, I64, P, P, P, P]),
     "aae_pad_weights_floats": (I64, [I, I]),
@@ -149,7 +150,7 @@ def last_error():
 
 
 # kernels launched per entry point (for the bench's gpu_launches claim); memcpy-only calls count 0
-KERNELS = {"aae_upload_batch": 0, "aae_w1_sweep_blocked": 2, "aae_batch_gather": 2, "aae_batch_corrupt": 2, "aae_rank_counts": 3, "aae_masked_topk": 2, "aae_predict_topk": 6, "aae_predict_topk2": 8, "aae_masked_topk_filtered": 3, "aae_predict_topk_filtered": 6,
+KERNELS = {"aae_upload_batch": 0, "aae_w1_sweep_blocked": 2, "aae_batch_gather": 2, "aae_batch_corrupt": 2, "aae_rank_counts": 3, "aae_rank_counts_filtered": 4, "aae_masked_topk": 2, "aae_predict_topk": 6, "aae_predict_topk2": 8, "aae_masked_topk_filtered": 3, "aae_predict_topk_filtered": 6,
            "aae_predict_topk2_filtered": 8, "aae_trace_set": 0, "aae_trace_slots": 0,
            "aae_peer_alloc": 0, "aae_peer_open": 0, "aae_peer_close": 0, "aae_peer_free": 0, "aae_peer_error": 0}
 TRACE_NAMES = ("batch_prepare", "w1_sweep_untouched", "ae_fwd", "dec_out_train", "ae_bwd", "ae_wgrad", "w1_rows_update_1",

@@ -9,6 +9,7 @@ defaults, ``fit`` / ``partial_fit`` / ``predict`` / ``eval`` / ``train`` / ``__s
 Additions that are not in the reference (defaults keep the reference's behaviour):
   ``predict_topk(X, k)``  fused predict + remove_non_missing + argtopk without the dense [n,V] matrix
   ``evaluate_topk(X, Y, metrics)``  the harness' ranking metrics (evaluation.py:70-164, 202-240) on the device
+  ``items=`` / ``exclude=``  candidate restriction of both: only eligible, non-excluded items are ranked
   ``rng='native'|'oracle'``  in-kernel Philox dropout / prior sampling, or the reference's CPU-generator
                            draws in the reference's order (bit-identical masks; used by parity tests)
   ``impl``  decoder-output kernel: 'auto', 'simt' (exact fp32 CUDA cores), 'tc' = 'parity' (tcgen05 3xTF32, fp32-accurate),
@@ -642,29 +643,53 @@ class AdversarialAutoEncoder(object):
             return np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts])
         return np.concatenate(parts)
 
-    def gold_ranks(self, X, Y, condition_data=None, batch_size=256):
+    def gold_ranks(self, X, Y, condition_data=None, batch_size=256, items=None, exclude=None):
         """Rank (1-based) of every held-out item of ``Y`` (scipy sparse [n, n_items], the harness' ``y_test``) in the
         ranking of remove_non_missing(predict(X), X): (indptr, ranks) aligned with ``Y.tocsr()``'s entries.  The score
-        matrix is built and ranked on the device batch by batch; only the ranks travel to the host."""
+        matrix is built and ranked on the device batch by batch; only the ranks travel to the host.
+
+        ``items`` / ``exclude`` (as in ``predict_topk``, same ValueErrors): the ranks are the 1-based positions in
+        the list ``predict_topk(X, None, items=items, exclude=exclude)`` returns.  A gold item that is ineligible or
+        excluded for its row is not in that list: its rank is 0."""
+        filt = RankFilter.build(self.engine.V, X.shape[0], items, exclude)
+        return self._gold_ranks(X, Y, condition_data, batch_size, filt)
+
+    def _gold_ranks(self, X, Y, condition_data, batch_size, filt):
         eng = self.engine
         Y = _canonical_csr(Y, "gold matrix")
-        assert Y.shape == (X.shape[0], eng.V), (Y.shape, X.shape, eng.V)
+        if Y.shape != (X.shape[0], eng.V):
+            raise ValueError("gold matrix has shape %s, expected (%d, %d)" % (Y.shape, X.shape[0], eng.V))
         ranks = np.zeros(Y.nnz, dtype=np.int64)
+        # returnable gold only go to the device; the others keep rank 0
+        keep = None if filt is None else filt.returnable(Y.indptr, Y.indices)
         scratch = torch.empty(min(batch_size, X.shape[0]), eng.Vloc, dtype=torch.float32, device=eng.dev)
         for start, end, B in self._iter_batches(X, condition_data, batch_size=batch_size):
             lo, hi = int(Y.indptr[start]), int(Y.indptr[end])
-            gp = (Y.indptr[start:end + 1] - lo).astype(np.int32)
-            ranks[lo:hi] = eng.gold_ranks(B, gp, Y.indices[lo:hi], scratch=scratch)
+            if keep is None:
+                gp = (Y.indptr[start:end + 1] - lo).astype(np.int32)
+                ranks[lo:hi] = eng.gold_ranks(B, gp, Y.indices[lo:hi], scratch=scratch)
+                continue
+            m = keep[lo:hi]
+            gp = np.concatenate(([0], np.cumsum(m)))[Y.indptr[start:end + 1] - lo].astype(np.int32)
+            ranks[lo:hi][m] = eng.gold_ranks(B, gp, Y.indices[lo:hi][m], scratch=scratch,
+                                             filt=filt.rows(start, end))
         eng.check_exchange()
         return Y.indptr.astype(np.int64), ranks
 
-    def evaluate_topk(self, X, Y, metrics, condition_data=None, batch_size=256):
+    def evaluate_topk(self, X, Y, metrics, condition_data=None, batch_size=256, items=None, exclude=None):
         """The harness' ``evaluate(y_test, remove_non_missing(predict(X), X), metrics)`` (evaluation.py:202-240, 395)
         without the dense [n, n_items] matrix ever reaching the host: [(mean, std)] per metric.  ``metrics``: keys of
-        evaluation.py:166-180 ('mrr@5', 'map', 'P@1' ...) or the reference's metric objects."""
+        evaluation.py:166-180 ('mrr@5', 'map', 'P@1' ...) or the reference's metric objects.
+
+        ``items`` / ``exclude`` (as in ``predict_topk``): the same metrics of the list ``predict_topk(X, None,
+        items=items, exclude=exclude)`` returns.  A gold item that is ineligible or excluded for its row is never a
+        hit and takes no place in MAP's count; a row whose gold are all such scores 0.  ``P`` without k divides by the
+        number of eligible items (the list's length)."""
         from .ranking import metrics_from_ranks
-        indptr, ranks = self.gold_ranks(X, Y, condition_data=condition_data, batch_size=batch_size)
-        return metrics_from_ranks(indptr, ranks, metrics, self.engine.V)
+        filt = RankFilter.build(self.engine.V, X.shape[0], items, exclude)
+        indptr, ranks = self._gold_ranks(X, Y, condition_data, batch_size, filt)
+        V = self.engine.V
+        return metrics_from_ranks(indptr, ranks, metrics, V if filt is None else filt.n_eligible(V))
 
 
 class AutoEncoder(AdversarialAutoEncoder):
@@ -750,9 +775,9 @@ class AAERecommender(Recommender):
         return self.model.predict_topk(X, k, condition_data=condition_data, mask_known=mask_known, items=items,
                                        exclude=exclude)
 
-    def evaluate_topk(self, test_set, gold, metrics):
+    def evaluate_topk(self, test_set, gold, metrics, items=None, exclude=None):
         """Ranking metrics of the harness (evaluation.py:70-164, 202-240) on the device: ``gold`` is the sparse
         [n, n_items] matrix of held-out items (``Evaluation.y_test``)."""
         X = test_set.tocsr()
         condition_data = self._condition_data(test_set, fit=False)
-        return self.model.evaluate_topk(X, gold, metrics, condition_data=condition_data)
+        return self.model.evaluate_topk(X, gold, metrics, condition_data=condition_data, items=items, exclude=exclude)

@@ -32,6 +32,8 @@ class Recommender(abc.ABC):
         ``items`` / ``exclude`` restrict the candidates (``AdversarialAutoEncoder.predict_topk``)."""
         raise NotImplementedError("%s ranks through predict() only" % type(self).__name__)
 
-    def evaluate_topk(self, test_set, gold, metrics):
-        """The harness' ranking metrics (evaluation.py:70-164, 202-240) computed from device-side ranks."""
+    def evaluate_topk(self, test_set, gold, metrics, items=None, exclude=None):
+        """The harness' ranking metrics (evaluation.py:70-164, 202-240) computed from device-side ranks; ``items`` /
+        ``exclude`` evaluate the candidate-restricted list of ``predict_topk``
+        (``AdversarialAutoEncoder.evaluate_topk``)."""
         raise NotImplementedError("%s evaluates through predict() only" % type(self).__name__)

@@ -129,3 +129,8 @@ class DAERecommender(Recommender):
         X = test_set.tocsr()
         return self.dae.predict_topk(X, k, condition_data=self._condition_data(test_set, fit=False),
                                      mask_known=mask_known, items=items, exclude=exclude)
+
+    def evaluate_topk(self, test_set, gold, metrics, items=None, exclude=None):
+        X = test_set.tocsr()
+        return self.dae.evaluate_topk(X, gold, metrics, condition_data=self._condition_data(test_set, fit=False),
+                                      items=items, exclude=exclude)

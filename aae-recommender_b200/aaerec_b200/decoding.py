@@ -151,3 +151,7 @@ class DecodingRecommender(Recommender):
         X, condition_data = self._query(test_set)
         return self.model.predict_topk(X, k, condition_data=condition_data, mask_known=mask_known, items=items,
                                        exclude=exclude)
+
+    def evaluate_topk(self, test_set, gold, metrics, items=None, exclude=None):
+        X, condition_data = self._query(test_set)
+        return self.model.evaluate_topk(X, gold, metrics, condition_data=condition_data, items=items, exclude=exclude)

@@ -1046,27 +1046,60 @@ class AAEEngine(object):
         return out
 
     @_on_device
-    def gold_ranks(self, B, gold_indptr, gold_indices, scratch=None, mask_known=True):
+    def gold_ranks(self, B, gold_indptr, gold_indices, scratch=None, mask_known=True, filt=None):
         """Ranks (1-based) of the gold items of the batch in the device buffers, in the descending order of
         remove_non_missing(predict(X), X) (known items at the bottom; ties by lower item id): int64 host array aligned
         with ``gold_indices``.  ``gold_indptr`` [B+1] / ``gold_indices``: CSR of the held-out items (global ids).
-        The [B, V] score matrix lives in HBM only (never on the host)."""
+        The [B, V] score matrix lives in HBM only (never on the host).
+
+        ``filt`` (``filters.RankFilter`` of the B rows): ranks in the full filtered ranking (``predict_topk(X, None,
+        items=, exclude=)``) -- only the eligible items, never an excluded (row, item) pair.  The caller passes only returnable gold
+        (eligible, not excluded for its row).  Each shard scores the compact copy of its eligible rows (``_compact``,
+        the copy ``topk`` ranks) into ``scratch`` and counts with ``aae_rank_counts_filtered``; a shard whose items are
+        all eligible counts on its own columns, with the exclusions only; a shard without an eligible item launches
+        neither but still takes part in the encoder exchange and both all-reduces."""
         n_gold = int(gold_indptr[-1])
         if n_gold == 0:
             return np.zeros(0, dtype=np.int64)
-        if scratch is None or scratch.shape[0] < B or scratch.shape[1] < self.Vloc:
-            scratch = torch.empty(B, self.Vloc, dtype=torch.float32, device=self.dev)
+        ids = excl = None
+        if filt is not None:
+            ids = filt.shard_ids(self.V, self.rank, self.world)
+            excl = filt.exclude if filt.exclude is not None and filt.exclude.nnz else None   # rows without any
         gp = torch.from_numpy(np.ascontiguousarray(gold_indptr, dtype=np.int32)).to(self.dev)
         gi = torch.from_numpy(np.ascontiguousarray(gold_indices, dtype=np.int32)).to(self.dev)
         zg = torch.empty(n_gold, dtype=torch.float32, device=self.dev)
         cnt = torch.zeros(n_gold, dtype=torch.int32, device=self.dev)
-        self.scores(B, scratch, apply_sigmoid=False)
+        if ids is None and excl is None:        # unfiltered, or every item of this shard eligible without exclusions
+            n, vb, fn, extra = self.Vloc, self.v_begin, "aae_rank_counts", ()
+            if scratch is None or scratch.shape[0] < B or scratch.shape[1] < n:
+                scratch = torch.empty(B, n, dtype=torch.float32, device=self.dev)
+            self.scores(B, scratch, apply_sigmoid=False)
+        else:
+            # first, on every path: on item shards predict_h2 is a collective (the h1pre exchange)
+            self.predict_h2(B)
+            if ids is not None and ids.size == 0:
+                n = 0
+                zg.fill_(float("nan"))          # no gold of this shard: contributes 0 to the summed scores
+            else:
+                if ids is None:
+                    W, b, n, vb, ids_dev = self.Wd3, self.bd3, self.Vloc, self.v_begin, None
+                else:
+                    c = self._compact(ids)
+                    W, b, n, vb, ids_dev = c["Wd3c"], c["bd3c"], c["A"], 0, c["ids"]
+                if scratch is None or scratch.shape[0] < B or scratch.shape[1] < n:
+                    scratch = torch.empty(B, n, dtype=torch.float32, device=self.dev)
+                call("aae_dec_out_scores", ptr(self.h2), B, self.H, ptr(W), ptr(b), n, 0, ptr(scratch),
+                     scratch.stride(0), self.impl_for_scores(), self._stream())
+                xp, xi = self._upload_exclusions(excl) if excl is not None else (None, None)
+                fn, extra = "aae_rank_counts_filtered", (C.byref(N.AaeRankFilter(ptr(ids_dev), ptr(xp), ptr(xi))),)
 
         def run(given):
-            call("aae_rank_counts", ptr(scratch), scratch.stride(0), B, self.Vloc, self.v_begin,
+            if n == 0:
+                return
+            call(fn, ptr(scratch), scratch.stride(0), B, n, vb,
                  ptr(self.indptr) if (mask_known and not given) else None,
                  ptr(self.indices) if (mask_known and not given) else None, ptr(gp), ptr(gi), n_gold, ptr(zg),
-                 1 if given else 0, ptr(cnt), self._stream())
+                 1 if given else 0, ptr(cnt), self._stream(), *extra)
         run(False)
         if self.world > 1:
             import torch.distributed as dist

@@ -81,3 +81,25 @@ class RankFilter(object):
 
     def n_eligible(self, V):
         return V if self.items is None else int(self.items.size)
+
+    def returnable(self, indptr, indices):
+        """bool mask of the entries of a CSR (rows = the query rows of this filter, sorted columns) whose item may be
+        returned for its row: eligible and not excluded.  The gold items of ``evaluate_topk`` that are not returnable
+        are not in the ranked list."""
+        indptr = np.asarray(indptr, dtype=np.int64)
+        indices = np.asarray(indices, dtype=np.int64)
+        ok = np.ones(indices.size, dtype=bool)
+        if self.items is not None:
+            pos = np.searchsorted(self.items, indices)
+            ok &= pos < self.items.size
+            ok[ok] = self.items[pos[ok]] == indices[ok]
+        if self.exclude is not None:
+            # intersection of the sorted rows of both CSRs, as ascending (row, item) keys
+            V, ex = self.exclude.shape[1], self.exclude
+            key = np.repeat(np.arange(indptr.size - 1, dtype=np.int64), np.diff(indptr)) * V + indices
+            ekey = np.repeat(np.arange(ex.shape[0], dtype=np.int64), np.diff(ex.indptr)) * V + ex.indices
+            pos = np.searchsorted(ekey, key)
+            hit = pos < ekey.size
+            hit[hit] = ekey[pos[hit]] == key[hit]
+            ok &= ~hit
+        return ok

@@ -31,15 +31,18 @@ def parse_metric(m):
 
 
 def per_row_metric(gold_indptr, ranks, kind, k, n_items):
-    """Per-row values of one metric; ``ranks`` (1-based) is aligned with the gold CSR entries."""
+    """Per-row values of one metric; ``ranks`` (1-based) is aligned with the gold CSR entries.  Rank 0 means "not in
+    the ranked list" (a gold item a candidate filter leaves out): it sorts after every ranked gold item of its row and
+    is never a hit.  ``n_items`` is the length of the ranked list (the denominator of P without k)."""
     gold_indptr = np.asarray(gold_indptr, dtype=np.int64)
     n = gold_indptr.shape[0] - 1
     ranks = np.asarray(ranks, dtype=np.int64)
     rows = np.repeat(np.arange(n), np.diff(gold_indptr))
-    order = np.lexsort((ranks, rows))
-    r, rows = ranks[order].astype(np.float64), rows[order]
+    absent = ranks <= 0
+    order = np.lexsort((np.where(absent, np.iinfo(np.int64).max, ranks), rows))
+    r, rows, absent = ranks[order].astype(np.float64), rows[order], absent[order]
     pos = np.arange(r.shape[0]) - gold_indptr[rows] + 1            # i of the i-th best gold item of its row
-    hit = np.ones(r.shape[0], dtype=bool) if k is None else (r <= k)
+    hit = ~absent if k is None else (~absent & (r <= k))
     out = np.zeros(n, dtype=np.float64)
     if kind == "mrr":
         first = pos == 1
@@ -47,7 +50,8 @@ def per_row_metric(gold_indptr, ranks, kind, k, n_items):
         out[rows[sel]] = 1.0 / r[sel]
     elif kind == "p":
         denom = float(n_items if k is None else k)
-        np.add.at(out, rows[hit], 1.0 / denom)
+        if denom:                   # 0: an empty list (no eligible item), which has no hit
+            np.add.at(out, rows[hit], 1.0 / denom)
     elif kind == "map":
         num = np.zeros(n, dtype=np.float64)
         cnt = np.zeros(n, dtype=np.float64)

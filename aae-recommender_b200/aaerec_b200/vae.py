@@ -122,6 +122,11 @@ class VAE(AutoEncoder):
         return super().predict_topk(X, k, condition_data=condition_data, mask_known=mask_known,
                                     return_scores=return_scores, shard=shard, items=items, exclude=exclude)
 
+    def _gold_ranks(self, X, Y, condition_data, batch_size, filt):
+        # gold_ranks and evaluate_topk: native noise, as in predict_topk (an oracle-RNG predict leaves its noise set)
+        self.engine.eval_injected = False
+        return super()._gold_ranks(X, Y, condition_data, batch_size, filt)
+
 
 class VAERecommender(Recommender):
     """Varietional Autoencoder Recommender (vae.py:269-340): same constructor, ``train`` / ``predict`` on Bags."""
@@ -163,3 +168,8 @@ class VAERecommender(Recommender):
         X = test_set.tocsr()
         return self.model.predict_topk(X, k, condition_data=self._condition_data(test_set, fit=False),
                                        mask_known=mask_known, items=items, exclude=exclude)
+
+    def evaluate_topk(self, test_set, gold, metrics, items=None, exclude=None):
+        X = test_set.tocsr()
+        return self.model.evaluate_topk(X, gold, metrics, condition_data=self._condition_data(test_set, fit=False),
+                                        items=items, exclude=exclude)

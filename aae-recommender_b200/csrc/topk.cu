@@ -583,10 +583,18 @@ static size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 //   gold_scores_kernel : zg[p] = scores[row(p), gold[p]]  (NaN when the item belongs to another shard)
 //   rank_count_kernel  : grid (column chunks, rows); each CTA counts, for up to RC_G gold items of its row at a
 //                        time, the entries of its column chunk that rank before them; one atomicAdd per CTA and gold.
+// The bodies take FILT: the columns are those of a filtered set (ids = ascending global id of each column, NULL:
+// v_begin + column).  The gold items stay global ids; a gold's tie position is then lb = lower_bound(ids, gold), the
+// number of columns with a lower id, so "column < lb" is "id < gold" also for a gold that is not a column.  The
+// unfiltered kernels instantiate FILT = false and keep their names; the *_filt_kernel ones instantiate FILT = true.
+// rank_count_body takes threadIdx.x from its kernel: read there, it carries the range the kernel's launch bounds give
+// it, so the FILT = false instantiation compiles to the code of the kernel before it was split.
 // ---------------------------------------------------------------------------------------------
-__global__ void gold_scores_kernel(const float* __restrict__ scores, int64_t lds, int B, int Vloc, int v_begin,
-                                   const int32_t* __restrict__ gold_indptr, const int32_t* __restrict__ gold_indices,
-                                   float* __restrict__ zg) {
+template <bool FILT>
+__device__ __forceinline__ void gold_scores_body(const float* __restrict__ scores, int64_t lds, int B, int Vloc,
+                                                 int v_begin, const int32_t* __restrict__ gold_indptr,
+                                                 const int32_t* __restrict__ gold_indices, float* __restrict__ zg,
+                                                 const int32_t* __restrict__ ids) {
   const int n = gold_indptr[B];
   for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {
     int lo = 0, hi = B;
@@ -594,34 +602,58 @@ __global__ void gold_scores_kernel(const float* __restrict__ scores, int64_t lds
       int mid = (lo + hi) >> 1;
       if (gold_indptr[mid + 1] <= e) lo = mid + 1; else hi = mid;
     }
-    const int i = gold_indices[e] - v_begin;
+    const int i = FILT ? col_of(ids, Vloc, v_begin, gold_indices[e]) : gold_indices[e] - v_begin;
     zg[e] = (i >= 0 && i < Vloc) ? scores[(size_t)lo * lds + i] : __int_as_float(0x7fc00000);
   }
 }
+__global__ void gold_scores_kernel(const float* __restrict__ scores, int64_t lds, int B, int Vloc, int v_begin,
+                                   const int32_t* __restrict__ gold_indptr, const int32_t* __restrict__ gold_indices,
+                                   float* __restrict__ zg) {
+  gold_scores_body<false>(scores, lds, B, Vloc, v_begin, gold_indptr, gold_indices, zg, nullptr);
+}
+__global__ void gold_scores_filt_kernel(const float* __restrict__ scores, int64_t lds, int B, int Vloc, int v_begin,
+                                        const int32_t* __restrict__ gold_indptr,
+                                        const int32_t* __restrict__ gold_indices, float* __restrict__ zg,
+                                        const int32_t* __restrict__ ids) {
+  gold_scores_body<true>(scores, lds, B, Vloc, v_begin, gold_indptr, gold_indices, zg, ids);
+}
 constexpr int RC_THREADS = 256, RC_G = 8, RC_CHUNK = 16384;
-__global__ void __launch_bounds__(RC_THREADS) rank_count_kernel(const float* __restrict__ scores, int64_t lds, int Vloc,
-                                                                int v_begin,
-                                                                const int32_t* __restrict__ gold_indptr,
-                                                                const int32_t* __restrict__ gold_indices,
-                                                                const float* __restrict__ zg,
-                                                                int32_t* __restrict__ cnt) {
-  __shared__ int red[RC_THREADS / 32][RC_G];
+template <bool FILT>
+__device__ __forceinline__ void rank_count_body(const float* __restrict__ scores, int64_t lds, int Vloc, int v_begin,
+                                                const int32_t* __restrict__ gold_indptr,
+                                                const int32_t* __restrict__ gold_indices,
+                                                const float* __restrict__ zg, int32_t* __restrict__ cnt,
+                                                const int32_t* __restrict__ ids, unsigned tid) {
+  __shared__ int red[RC_THREADS / 32 + (FILT ? 1 : 0)][RC_G];    // FILT: the last row holds the gold tie positions
+  int* lb_s = red[RC_THREADS / 32];
   const int row = blockIdx.y;
   const int c0 = blockIdx.x * RC_CHUNK, c1 = min(Vloc, c0 + RC_CHUNK);
   const int p0 = gold_indptr[row], p1 = gold_indptr[row + 1];
   const float* r = scores + (size_t)row * lds;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int lane = tid & 31, warp = tid >> 5;
   for (int g0 = p0; g0 < p1; g0 += RC_G) {
+    if (FILT && ids) {          // tie position of each gold of the group, once per CTA (ids is uniform: no divergence)
+      if (tid < RC_G && g0 + tid < p1) {
+        const int g = gold_indices[g0 + tid];
+        int lo = 0, hi = Vloc;
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (__ldg(ids + mid) < g) lo = mid + 1; else hi = mid;
+        }
+        lb_s[tid] = lo;
+      }
+      __syncthreads();
+    }
     float z[RC_G];
     int id[RC_G], c[RC_G];
 #pragma unroll
     for (int j = 0; j < RC_G; ++j) {
       const bool ok = g0 + j < p1;
       z[j] = ok ? zg[g0 + j] : __int_as_float(0x7fc00000);      // NaN compares false: counts stay 0
-      id[j] = ok ? gold_indices[g0 + j] - v_begin : -1;
+      id[j] = ok ? ((FILT && ids) ? lb_s[j] : gold_indices[g0 + j] - v_begin) : -1;
       c[j] = 0;
     }
-    for (int v = c0 + threadIdx.x; v < c1; v += RC_THREADS) {
+    for (int v = c0 + tid; v < c1; v += RC_THREADS) {
       const float x = r[v];
 #pragma unroll
       for (int j = 0; j < RC_G; ++j) c[j] += (x > z[j] || (x == z[j] && v < id[j])) ? 1 : 0;
@@ -633,13 +665,30 @@ __global__ void __launch_bounds__(RC_THREADS) rank_count_kernel(const float* __r
       if (lane == 0) red[warp][j] = t;
     }
     __syncthreads();
-    if (threadIdx.x < RC_G && g0 + threadIdx.x < p1) {
+    if (tid < RC_G && g0 + tid < p1) {
       int t = 0;
-      for (int w = 0; w < RC_THREADS / 32; ++w) t += red[w][threadIdx.x];
-      if (t) atomicAdd(cnt + g0 + threadIdx.x, t);
+      for (int w = 0; w < RC_THREADS / 32; ++w) t += red[w][tid];
+      if (t) atomicAdd(cnt + g0 + tid, t);
     }
     __syncthreads();
   }
+}
+__global__ void __launch_bounds__(RC_THREADS) rank_count_kernel(const float* __restrict__ scores, int64_t lds, int Vloc,
+                                                                int v_begin,
+                                                                const int32_t* __restrict__ gold_indptr,
+                                                                const int32_t* __restrict__ gold_indices,
+                                                                const float* __restrict__ zg,
+                                                                int32_t* __restrict__ cnt) {
+  rank_count_body<false>(scores, lds, Vloc, v_begin, gold_indptr, gold_indices, zg, cnt, nullptr, threadIdx.x);
+}
+__global__ void __launch_bounds__(RC_THREADS) rank_count_filt_kernel(const float* __restrict__ scores, int64_t lds,
+                                                                     int Vloc, int v_begin,
+                                                                     const int32_t* __restrict__ gold_indptr,
+                                                                     const int32_t* __restrict__ gold_indices,
+                                                                     const float* __restrict__ zg,
+                                                                     int32_t* __restrict__ cnt,
+                                                                     const int32_t* __restrict__ ids) {
+  rank_count_body<true>(scores, lds, Vloc, v_begin, gold_indptr, gold_indices, zg, cnt, ids, threadIdx.x);
 }
 
 }  // namespace aae
@@ -753,6 +802,42 @@ int aae_rank_counts(float* scores, int64_t lds, int B, int Vloc, int v_begin, co
   dim3 grid((unsigned)cdiv(Vloc, RC_CHUNK), (unsigned)B);
   rank_count_kernel<<<grid, RC_THREADS, 0, s>>>(scores, lds, Vloc, v_begin, gold_indptr, gold_indices, gold_scores,
                                                 counts);
+  return check_launch("rank_count");
+}
+
+int aae_rank_counts_filtered(float* scores, int64_t lds, int B, int Vloc, int v_begin, const int32_t* indptr,
+                             const int32_t* indices, const int32_t* gold_indptr, const int32_t* gold_indices,
+                             int n_gold, float* gold_scores, int gold_scores_given, int32_t* counts, void* stream,
+                             const aae_rank_filter* filt) {
+  if (!filter_active(filt))
+    return aae_rank_counts(scores, lds, B, Vloc, v_begin, indptr, indices, gold_indptr, gold_indices, n_gold,
+                           gold_scores, gold_scores_given, counts, stream);
+  AAE_REQUIRE(scores && gold_indptr && gold_indices && gold_scores && counts, "null pointer");
+  AAE_REQUIRE(B > 0 && Vloc > 0 && n_gold >= 0 && lds >= Vloc, "bad size");
+  int rc = check_filter(filt, v_begin, __func__);
+  if (rc) return rc;
+  cudaStream_t s = as_stream(stream);
+  const int grid = std::min(4 * sm_count(), std::max(1, cdiv((int64_t)B * 32, 256)));
+  if (indptr && indices) {
+    mask_cols_kernel<<<grid, 256, 0, s>>>(scores, lds, B, Vloc, v_begin, filt->item_ids, indptr, indices, -FLT_MAX);
+    rc = check_launch("mask_cols(known)");
+    if (rc) return rc;
+  }
+  // excluded entries at -inf never rank before a returnable gold, whose score is finite (-FLT_MAX when known)
+  if (filt->excl_indptr) {
+    mask_cols_kernel<<<grid, 256, 0, s>>>(scores, lds, B, Vloc, v_begin, filt->item_ids, filt->excl_indptr,
+                                          filt->excl_indices, -INFINITY);
+    rc = check_launch("mask_cols(exclude)");
+    if (rc) return rc;
+  }
+  if (n_gold == 0) return AAE_OK;
+  cudaMemsetAsync(counts, 0, sizeof(int32_t) * (size_t)n_gold, s);
+  if (!gold_scores_given)
+    gold_scores_filt_kernel<<<std::min(4 * sm_count(), std::max(1, cdiv(n_gold, 256))), 256, 0, s>>>(
+        scores, lds, B, Vloc, v_begin, gold_indptr, gold_indices, gold_scores, filt->item_ids);
+  dim3 rgrid((unsigned)cdiv(Vloc, RC_CHUNK), (unsigned)B);
+  rank_count_filt_kernel<<<rgrid, RC_THREADS, 0, s>>>(scores, lds, Vloc, v_begin, gold_indptr, gold_indices,
+                                                      gold_scores, counts, filt->item_ids);
   return check_launch("rank_count");
 }
 

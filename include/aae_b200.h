@@ -365,6 +365,21 @@ int aae_predict_topk2_filtered(const float* h2, int B, int H, const float* Wd3, 
 int aae_rank_counts(float* scores, int64_t lds, int B, int Vloc, int v_begin, const int32_t* indptr,
                     const int32_t* indices, const int32_t* gold_indptr, const int32_t* gold_indices, int n_gold,
                     float* gold_scores, int gold_scores_given, int32_t* counts, void* stream);
+/* aae_rank_counts on a filtered column set (evaluate_topk(..., items=, exclude=)): the gold ranks in the list that
+ * aae_predict_topk*_filtered / aae_masked_topk_filtered return in full.  scores [B, >=Vloc] are the logits of the
+ * filter's columns: the compact copy of aae_gather_item_rows when filt->item_ids is set (then v_begin must be 0), else
+ * the shard's own columns v_begin + c.  Known items that are columns become -FLT_MAX, excluded (row, item) pairs
+ * -INFINITY, so an excluded item never ranks before a gold.  The caller passes only returnable gold: items that are
+ * eligible and not excluded for their row (on some shard); their rank in the filtered list is 1 + the counts summed
+ * over item shards.  Gold items stay global ids.  With a column table a gold's tie position is the number of columns
+ * with a lower id (a lower bound in item_ids), so the lower-id tie rule holds for a gold of another shard as well;
+ * its score is that of its column, or NaN when it is not a column of this shard (the two-pass protocol of
+ * aae_rank_counts then applies unchanged: NaN -> 0, sum over shards, call again with gold_scores_given != 0).  A NULL
+ * filter, or one with both tables NULL, is exactly aae_rank_counts. */
+int aae_rank_counts_filtered(float* scores, int64_t lds, int B, int Vloc, int v_begin, const int32_t* indptr,
+                             const int32_t* indices, const int32_t* gold_indptr, const int32_t* gold_indices,
+                             int n_gold, float* gold_scores, int gold_scores_given, int32_t* counts, void* stream,
+                             const aae_rank_filter* filt);
 
 /* ---- device-side epoch feed --------------------------------------------------------------------
  * Replaces sklearn.utils.shuffle(X, *condition_data) + X_shuf[start:end].toarray() (aae.py:815-823) and the
